@@ -169,7 +169,8 @@ class NvmlSampler:
 
 # ------------------------------------------------------------------------------------------------ CPU / reference legs
 def cpu_reference_rate(encoder, size, steps, warmup):
-    """Times the oracle (CPU restatement of the reference forward) on all host cores: `steps` images, ONE image per step."""
+    """Times the oracle (CPU restatement of the reference forward) on all host cores: `steps` images, ONE image per step.
+    Returns (images/s, s/image, threads, output of the last step)."""
     import torch
     from oracle import amodal_oracle as O
     from oracle import synth
@@ -179,11 +180,11 @@ def cpu_reference_rate(encoder, size, steps, warmup):
     times = []
     for i in range(warmup + steps):
         t0 = time.perf_counter()
-        O.forward(sd, encoder, GT, inp["x"], None, inp["guide_mask"], inp["observation"])
+        out = O.forward(sd, encoder, GT, inp["x"], None, inp["guide_mask"], inp["observation"])
         if i >= warmup:
             times.append(time.perf_counter() - t0)
     sec = sum(times) / len(times)
-    return 1.0 / sec, sec, torch.get_num_threads()
+    return 1.0 / sec, sec, torch.get_num_threads(), out
 
 
 def cpu_context():
@@ -196,7 +197,7 @@ def cpu_context():
                 break
     except OSError:
         pass
-    _, sec_s, _ = cpu_reference_rate("vits", 518, 5, 1)
+    _, sec_s, _, _ = cpu_reference_rate("vits", 518, 5, 1)
     return {"cpu_model": model, "os_cpu_count": os.cpu_count(), "vits_518_b1_s_per_image": sec_s}
 
 
@@ -207,7 +208,12 @@ def run_reference(a):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    rate, sec, cores = cpu_reference_rate(a.encoder, a.size, a.steps, a.warmup)
+    rate, sec, cores, out = cpu_reference_rate(a.encoder, a.size, a.steps, a.warmup)
+    dumped = None
+    if a.dump_outputs:
+        import torch
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        dumped = dump_outputs(torch, out, os.path.join(a.dump_outputs, "depth.npy"), DUMP_BYTES)
     sample = (f"{a.steps} steps x 1 image per step ({a.encoder} {a.size}x{a.size}, fp32, torch CPU, {cores} threads) after "
               f"{a.warmup} warm-up; NOT the {a.batch}-image step of the GPU arm")
     cfg = workload_config(a, a.gpus)
@@ -220,6 +226,7 @@ def run_reference(a):
         "cpu_baseline": {"value": rate, "unit": "images/s", "cores": cores, "kind": "port", "sample": sample},
         "e2e": {"value": rate, "unit": "images/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
+        "dump_outputs": dumped,
     }
     print(json.dumps(line), flush=True)
 
@@ -360,6 +367,26 @@ def measure_config(torch, pkg, dev, encoder, size, batch, steps, warmup, peaks, 
     return r
 
 
+DUMP_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(torch, out, path, max_bytes):
+    """Writes the depth map a caller of the timed path receives to `path` (.npy, float32) for output-by-output comparison
+    of two builds. An output larger than `max_bytes` is replaced by a fixed, seeded sample of its elements (flat, in
+    index order), so two runs with the same arguments write the same elements."""
+    import numpy as np
+    a = out.detach().float().cpu().flatten()
+    cap = max_bytes // 4
+    if a.numel() > cap:
+        idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+        a = a[idx]
+    else:
+        a = a.view(out.shape)
+    np.save(path, a.numpy())
+    return {"file": os.path.basename(path), "shape": list(out.shape), "dtype": "float32", "elements": a.numel(),
+            "sampled": a.numel() < out.numel()}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -379,7 +406,12 @@ def main():
                          "0.7 ms per step slower at batch 32 and exposed to host-side launch stalls)")
     ap.add_argument("--profile-steps", type=int, default=2)
     ap.add_argument("--detail", default="", help="write per-launch-signature timings of the profile pass to this JSON file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the output of the last timed step to DIR/depth.npy (float32; "
+                         "depth_rank<r>.npy per rank with several GPUs; a fixed seeded sample above 64 MB in all)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(a.warmup, 3) if a.impl == "b200" else a.warmup
     a.graph = not a.no_graph
     if a.impl == "reference":
@@ -444,6 +476,11 @@ def main():
     ms = max_over_ranks(ms, dev)
     launches = model.launch_count()
     assert torch.isfinite(out).all()
+    dumped = None
+    if a.dump_outputs:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        name = "depth.npy" if world == 1 else f"depth_rank{rank}.npy"
+        dumped = dump_outputs(torch, out, os.path.join(a.dump_outputs, name), DUMP_BYTES // world)
 
     # ---- end to end through the public API: pinned host inputs -> H2D -> forward -> D2H, every step
     hx, hm, ho = x.cpu().pin_memory(), mask.cpu().pin_memory(), obs.cpu().pin_memory()
@@ -569,7 +606,7 @@ def main():
             other.append(measure_config(torch, pkg, dev, "vitl", 1036, 4, 5, 3, peaks, model=model))
     cpu_base = None
     if rank == 0 and world == 1 and not a.no_cpu_baseline:
-        rate, sec, cores = cpu_reference_rate(a.encoder, a.size, 3, 1)
+        rate, sec, cores, _ = cpu_reference_rate(a.encoder, a.size, 3, 1)
         cpu_base = {"context": cpu_context(), "value": rate, "unit": "images/s", "cores": cores, "kind": "port",
                     "sample": f"3 images of the same workload ({a.encoder} {a.size}x{a.size}, ONE image per step, fp32 torch CPU "
                               f"oracle) after 1 warm-up, {sec:.2f} s/image"}
@@ -604,6 +641,7 @@ def main():
             "other_configs": other or None,
             "cpu_baseline": cpu_base,
             "workspace_gb": workspace_gb,
+            "dump_outputs": dumped,
         }
         if eager:
             for k in ("fp32_no_tf32", "bf16_autocast"):

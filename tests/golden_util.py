@@ -20,7 +20,12 @@ def raw_golden_names():
 
 
 def load_golden(name, sub=""):
-    z = np.load(os.path.join(GOLDEN_DIR, sub, name + ".npz"))
+    """(meta, {key: array}). A fixture may hold its float32 output as the four little-endian byte planes
+    `output_planes` [4, *shape] (make_golden.py:byte_planes) instead of `output`; it is returned as `output`."""
+    with np.load(os.path.join(GOLDEN_DIR, sub, name + ".npz")) as f:
+        z = {k: f[k] for k in f.files}
+    if "output_planes" in z:
+        z["output"] = np.ascontiguousarray(np.moveaxis(z.pop("output_planes"), 0, -1)).view("<f4")[..., 0]
     meta = ast.literal_eval(str(z["meta"]))
     return meta, z
 

@@ -36,11 +36,43 @@ def test_reference_arm_other_ranks_exit_quietly():
 
 
 def test_product_arm_refuses_to_run_without_a_gpu():
-    import torch
-    if torch.cuda.is_available():
-        return
-    r = _run(["--steps", "1"])
+    r = _run(["--steps", "1"], {"CUDA_VISIBLE_DEVICES": ""})   # no visible device, also on a GPU machine
     assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
+
+
+def test_steps_below_one_are_refused():
+    r = _run(["--impl", "reference", "--encoder", "vits", "--size", "126", "--steps", "0", "--warmup", "0"])
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
+def test_reference_arm_dumps_the_same_last_step_output_every_run(tmp_path):
+    import numpy as np
+    got = []
+    for run in ("a", "b"):
+        r = _run(["--impl", "reference", "--encoder", "vits", "--size", "126", "--steps", "2", "--warmup", "0",
+                  "--dump-outputs", str(tmp_path / run)])
+        assert r.returncode == 0, r.stderr[-2000:]
+        d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+        assert d["steps"] == 2 and d["dump_outputs"]["file"] == "depth.npy" and not d["dump_outputs"]["sampled"]
+        got.append(np.load(tmp_path / run / "depth.npy"))
+    assert got[0].dtype == np.float32 and got[0].shape == (1, 1, 126, 126) and np.isfinite(got[0]).all()
+    assert np.array_equal(got[0], got[1])
+
+
+def test_dump_outputs_samples_a_large_output_the_same_way_every_time(tmp_path):
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    out = torch.arange(1000, dtype=torch.float32).view(10, 1, 10, 10)
+    info = bench.dump_outputs(torch, out, str(tmp_path / "a.npy"), 400)
+    bench.dump_outputs(torch, out, str(tmp_path / "b.npy"), 400)
+    a = np.load(tmp_path / "a.npy")
+    assert info["sampled"] and info["elements"] == 100 and info["shape"] == [10, 1, 10, 10]
+    assert a.dtype == np.float32 and a.nbytes <= 400 and a.shape == (100,)
+    assert np.array_equal(a, np.load(tmp_path / "b.npy")) and (np.diff(a) > 0).all()   # distinct elements, index order
+    info = bench.dump_outputs(torch, out, str(tmp_path / "c.npy"), 4000)
+    assert not info["sampled"] and np.array_equal(np.load(tmp_path / "c.npy"), out.numpy())
 
 
 def test_nvml_sampler_report_with_a_fake_nvml(monkeypatch):

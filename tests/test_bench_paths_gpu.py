@@ -130,6 +130,32 @@ def test_alternating_batch_sizes_on_a_side_stream_match_default_stream_results()
         assert torch.equal(o.cpu(), want[n]), n
 
 
+def test_bench_dump_is_the_last_timed_step_and_steps_sets_the_timed_steps(tmp_path):
+    """bench.py --dump-outputs writes what the timed path returned in its last step: the same numbers as a direct call of
+    the model on bench.py's own seeded weights and inputs. --steps is the number of timed steps."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import numpy as np
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--encoder", "vits", "--size", "126", "--batch", "2",
+                        "--steps", "3", "--warmup", "1", "--no-extras", "--no-cpu-baseline", "--profile-steps", "0",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+    assert d["steps"] == 3 and len(d["ms_steps_rank0"]) == 3 and d["dump_outputs"]["file"] == "depth.npy"
+    got = np.load(tmp_path / "depth.npy")
+    sys.path.insert(0, root)
+    import bench
+    dev = torch.device("cuda", 0)
+    m = bench.make_model(pkg, torch, "vits", dev)
+    x, mask, obs = bench.make_inputs(torch, 2, 126, 126, dev, 1234)
+    want = m(x, guide_rgb=None, guide_mask=mask, observation=obs).cpu().numpy()
+    assert got.dtype == np.float32 and got.shape == (2, 1, 126, 126)
+    assert np.array_equal(got, want)
+
+
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs in one process")
 def test_one_process_two_devices():
     """One process driving two GPUs, one model each (SURVEY.md section 5 "one process, N streams"): the per-kernel

@@ -81,7 +81,7 @@ def test_forward_matches_reference_golden(name):
     assert out.shape == ref.shape and out.dtype == torch.float32
     assert torch.isfinite(out).all()
     report = {}
-    for key in z.files:  # module-level parity points (SURVEY.md section 4), strided samples
+    for key in z:  # module-level parity points (SURVEY.md section 4), strided samples
         if not key.startswith("s_"):
             continue
         k = key[2:]
@@ -92,7 +92,7 @@ def test_forward_matches_reference_golden(name):
         scale = float(np.abs(z[key]).max())
         report[k] = float(np.abs(g - z[key]).max() / scale)
         assert report[k] < INTER_TOL[_inter_kind(k)], (k, report)
-    if "s_logits" in z.files and "ssi" not in meta["loss_stategy"]:
+    if "s_logits" in z and "ssi" not in meta["loss_stategy"]:
         # pre-sigmoid logits (dpt.py:195, output_conv2[2]) recovered from the fp32 output: logit = log(o / (1 - o))
         lg = sample(torch.log(out.double() / (1.0 - out.double())).float())
         report["logits_abs"] = float(np.abs(lg - z["s_logits"]).max())

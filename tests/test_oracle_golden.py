@@ -24,7 +24,7 @@ def test_oracle_matches_reference_golden(name):
     assert out.shape == ref.shape == (meta["B"], 1, meta["H"], meta["W"])
     # same ATen ops on the same CPU; only thread-count dependent summation order may differ -> 2e-5 absolute
     assert (out - ref).abs().max().item() < 2e-5
-    for key in z.files:
+    for key in z:
         if not key.startswith("s_"):
             continue
         k = key[2:]

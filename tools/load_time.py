@@ -1,4 +1,4 @@
-import sys, time; sys.path.insert(0,'/root/repo')
+import os, sys, time; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch, amodal_depth_anything_b200 as pkg
 for enc in ("vitl","vitg"):
     m = pkg.AmodalDAv2(guide_type="mask+observation", encoder=enc, pretrained=False).cuda().eval()
