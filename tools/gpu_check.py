@@ -392,6 +392,406 @@ def chk_gemm_resid_f32(M, N, K, gamma=True, cg=0):
     return _cmp("resid_f32", out, ref, 2e-3, 2e-3)
 
 
+# ---- implicit-GEMM conv: every pixel-tile shape and every epilogue the model launches, against an fp64 reference
+#
+# Error model. The kernels multiply bf16 operands exactly and accumulate in fp32, so an output before its final rounding is
+# off the fp64 result by less than 2^-16 * S, S = conv(|x|, |w|) + |b| (+ |r1| + |r2|): fp32 accumulation over K <= 9 * 1536
+# terms with room to spare. The output rounding adds at most one unit roundoff of the stored type: 2^-8 |ref| for bf16,
+# 2^-11 for fp16 (held to 2^-10), 2^-24 for fp32 (held to 2^-22: the epilogue rounds twice). The channel-LayerNorm
+# epilogue scales a pre-normalisation error by |LN weight| * rstd; its mean carries the channel average of the errors.
+REL_BF16, REL_F16, REL_F32, REL_ACC = 2.0 ** -8, 2.0 ** -10, 2.0 ** -22, 2.0 ** -16
+
+# One row per pixel-tile geometry (lw, lh, lb, pair) = 2^lw x 2^lh pixels of 2^lb images, CTA pairs side by side in x: all
+# 25 shapes with lw + lh + lb = 7, 1 <= lw <= 5, single and paired. (B, H, W) is a small map for which pick_tile_geo
+# (ada_conv_tile_shape) picks that shape, ragged in x, y and the batch wherever the shape has more than one pixel / image in
+# that direction; for the stride-2 variant it is the OUTPUT size. Cin 48 / 96 leave a ragged 64-channel chunk that the
+# packed weights zero-pad; N 48 / 96 are ragged N tiles whose stores are clipped. ada_op_gemm pairs CTAs on force_cg=2 only
+# for BN = 256 (or BN = 128 with the plain bf16 epilogue), so every paired row has N = 256, for which pick_bn picks 256.
+#   (lw, lh, lb, pair,  B,  H,  W, Cin,   N)
+CONV_GEO_ROWS = [
+    (1, 0, 6, 1, 33,  1,  1,  48,  48),
+    (1, 1, 5, 1, 25,  5,  5,  64,  96),
+    (1, 2, 4, 1, 25, 11,  5,  96, 128),
+    (1, 3, 3, 1, 13, 21,  5, 256, 256),
+    (1, 4, 2, 1,  7, 41,  5,  64,  48),
+    (1, 5, 1, 1,  5, 25,  5,  96,  96),
+    (1, 6, 0, 1,  3, 41,  9, 256, 128),
+    (2, 0, 5, 1, 25,  3,  9,  48, 256),
+    (2, 1, 4, 1, 37,  5,  3,  96,  48),
+    (2, 2, 3, 1, 13, 11, 11, 256,  96),
+    (2, 3, 2, 1,  7, 21, 11,  48, 128),
+    (2, 4, 1, 1,  5, 41, 11,  64, 256),
+    (2, 5, 0, 1,  3, 41,  3, 256,  48),
+    (3, 0, 4, 1, 25,  3, 21,  48,  96),
+    (3, 1, 3, 1, 21,  5, 21,  64, 128),
+    (3, 2, 2, 1,  7, 11, 21,  96, 256),
+    (3, 3, 1, 1,  5, 21, 21,  48,  48),
+    (3, 4, 0, 1,  2, 25, 23,  64,  96),
+    (4, 0, 3, 1, 13,  3, 41,  96, 128),
+    (4, 1, 2, 1, 10,  5, 41, 256, 256),
+    (4, 2, 1, 1,  5,  9, 41,  64,  48),
+    (4, 3, 0, 1,  2, 15, 29,  96,  96),
+    (5, 0, 2, 1,  7,  3, 49, 256, 128),
+    (5, 1, 1, 1,  5,  5, 49,  48, 256),
+    (5, 2, 0, 1,  2, 11, 49,  96,  48),
+    (1, 0, 6, 2, 33,  1,  1,  48, 256),
+    (1, 1, 5, 2, 25,  5,  9,  64, 256),
+    (1, 2, 4, 2, 25, 11,  9,  96, 256),
+    (1, 3, 3, 2, 13, 21,  9, 256, 256),
+    (1, 4, 2, 2,  7, 41,  9,  48, 256),
+    (1, 5, 1, 2,  5, 25,  9,  64, 256),
+    (1, 6, 0, 2,  3, 41, 17,  96, 256),
+    (2, 0, 5, 2, 25,  3, 17, 256, 256),
+    (2, 1, 4, 2, 37,  5,  5,  48, 256),
+    (2, 2, 3, 2, 13, 11,  5,  64, 256),
+    (2, 3, 2, 2,  7, 21,  5,  96, 256),
+    (2, 4, 1, 2,  5, 33,  5, 256, 256),
+    (2, 5, 0, 2,  3, 41,  5,  48, 256),
+    (3, 0, 4, 2, 25,  3,  9,  64, 256),
+    (3, 1, 3, 2, 19,  5,  9,  96, 256),
+    (3, 2, 2, 2,  7, 11,  9, 256, 256),
+    (3, 3, 1, 2,  5, 17,  9,  48, 256),
+    (3, 4, 0, 2,  2, 25, 45,  64, 256),
+    (4, 0, 3, 2, 13,  3, 21,  96, 256),
+    (4, 1, 2, 2, 10,  5, 17, 256, 256),
+    (4, 2, 1, 2,  5,  9, 17,  48, 256),
+    (4, 3, 0, 2,  2, 15, 57,  64, 256),
+    (5, 0, 2, 2,  7,  3, 41,  96, 256),
+    (5, 1, 1, 2,  5,  5, 33, 256, 256),
+    (5, 2, 0, 2,  3,  9, 33,  48, 256),
+]
+
+# The conv epilogues of the model's forward (csrc/ada_api.cu), each checked at every row:
+CONV_VARIANTS = {
+    "a_bias": dict(bias=True),                                # input_projection conv with C > 256; stride-1 plain conv
+    "b_relu_copy": dict(bias=False, relu_copy=True),          # layer_rn: no bias, keeps x and relu(x)
+    "c_relu": dict(bias=True, act="relu"),                    # RCU conv1
+    "d_resid2_relu_copy": dict(bias=True, resid=2, relu_copy=True),  # RCU1 conv2: + layer_rn + path, and its ReLU
+    "e_resid1": dict(bias=True, resid=1),                     # RCU2 conv2
+    "f_chln": dict(bias=True, epi="chln"),                    # input_projection with C <= 256: conv + channel LN + ReLU
+    "g_f16": dict(bias=True, epi="f16"),                      # output_conv1, stored as fp16 for the tail
+    "h_s2_bias": dict(bias=True, stride=2),                   # resize_layers[3]: stride 2
+}
+
+
+def conv_geo_operands(B, H, W, Cin, N, seed, s2_odd=True, device="cpu", variants=tuple(CONV_VARIANTS)):
+    """Operands of one table row: x NHWC [B, H, W, Cin] and xs (input of the stride-2 variant, (2H - 1) x (2W - 1) if
+    s2_odd else 2H x 2W) in bf16, weights [N, Cin, 3, 3] rounded to bf16 (held as fp32, so packing is exact), fp32 bias,
+    bf16 residuals [B, H, W, N], fp32 LayerNorm weight / bias. Maps no listed variant reads are left out."""
+    import torch
+    g = torch.Generator(device=device).manual_seed(seed)
+    Hs, Ws = (2 * H - 1, 2 * W - 1) if s2_odd else (2 * H, 2 * W)
+    vs = [CONV_VARIANTS[v] for v in variants]
+    rnd = lambda *s: torch.randn(*s, generator=g, device=device)  # noqa: E731
+    op = {
+        "w": (rnd(N, Cin, 3, 3) / (3 * Cin ** 0.5)).bfloat16().float(),
+        "b": rnd(N) * 0.1,
+        "lnw": 1.0 + 0.2 * rnd(N),
+        "lnb": 0.3 * rnd(N),
+    }
+    if any(v.get("stride", 1) == 1 for v in vs):
+        op["x"] = rnd(B, H, W, Cin).bfloat16()
+    if any(v.get("stride", 1) == 2 for v in vs):
+        op["xs"] = rnd(B, Hs, Ws, Cin).bfloat16()
+    for k in range(max(v.get("resid", 0) for v in vs)):
+        op[("r1", "r2")[k]] = rnd(B, H, W, N).bfloat16()
+    return op
+
+
+def conv_ref64(op, variant, imgs=None):
+    """fp64 reference of one epilogue variant on the operands of conv_geo_operands (any device): (ref, bound, relu_copy)
+    as [b, H, W, N] fp64 over the images `imgs` (all if None); bound is the per-element error bound of the error model
+    above, relu_copy whether the variant also stores relu(out)."""
+    import torch
+    F = torch.nn.functional
+    v = CONV_VARIANTS[variant]
+    stride = v.get("stride", 1)
+    x = op["xs"] if stride == 2 else op["x"]
+    sel = (lambda t: t) if imgs is None else (lambda t: t[list(imgs)])
+    xd = sel(x).double().permute(0, 3, 1, 2)
+    wd = op["w"].double()
+    acc = F.conv2d(xd, wd, stride=stride, padding=1).permute(0, 2, 3, 1)
+    S = F.conv2d(xd.abs(), wd.abs(), stride=stride, padding=1).permute(0, 2, 3, 1)
+    if v.get("bias"):
+        acc = acc + op["b"].double()
+        S = S + op["b"].double().abs()
+    if v.get("act") == "relu":
+        acc = torch.relu(acc)
+    for k in range(v.get("resid", 0)):
+        r = sel(op[("r1", "r2")[k]]).double()
+        acc = acc + r
+        S = S + r.abs()
+    if v.get("epi") == "chln":
+        mean = acc.mean(-1, keepdim=True)
+        rstd = 1.0 / torch.sqrt((acc - mean).pow(2).mean(-1, keepdim=True) + 1e-6)
+        lnw = op["lnw"].double()
+        ref = torch.relu((acc - mean) * rstd * lnw + op["lnb"].double())
+        bound = REL_BF16 * ref.abs() + REL_ACC * (S + S.mean(-1, keepdim=True)) * lnw.abs() * rstd
+        return ref, bound, False
+    rel = REL_F16 if v.get("epi") == "f16" else REL_BF16
+    return acc, rel * acc.abs() + REL_ACC * S, bool(v.get("relu_copy"))
+
+
+def relu_copy_of(out):
+    """What the ReLU copy must hold, bit for bit: clamp_min(out, 0), with -0 stored as +0."""
+    return (out.float().clamp_min(0) + 0.0).to(out.dtype)
+
+
+def err_over_bound(got, ref, bound):
+    """Largest |got - ref| / bound (inf if got has a NaN or an infinity)."""
+    import torch
+    err = (got.to(ref.device).double() - ref).abs()
+    q = torch.where(err == 0, torch.zeros_like(err), err / bound)
+    return float(q.nan_to_num(float("inf")).max().item())
+
+
+def conv_verdict(got, got_relu, ref, bound, relu_copy):
+    """Judges one variant's output(s) (already restricted to the reference's images): within the bound everywhere, no NaN
+    (an unwritten pixel of the NaN-filled buffer), and the ReLU copy exactly relu_copy_of(out)."""
+    import torch
+    r = {"err_bound": err_over_bound(got, ref, bound), "nan": int(torch.isnan(got.float()).sum().item())}
+    r["ok"] = r["err_bound"] <= 1.0 and r["nan"] == 0
+    if relu_copy:
+        r["relu_copy_exact"] = bool(torch.equal(got_relu.view(torch.int16), relu_copy_of(got).view(torch.int16)))
+        r["ok"] = r["ok"] and r["relu_copy_exact"]
+    return r
+
+
+class Guarded:
+    """A tensor inside a larger 1-D buffer: `guard` elements (a multiple of 64, so the tensor keeps TMA's 16-byte alignment)
+    before and after it. fill=None writes a fixed canary pattern into the guards (outputs: a store past the tensor changes
+    it); a float fill fills the guards with it (inputs: NaN, so a read past the tensor reaches the output)."""
+
+    def __init__(self, shape, dtype, device, guard, fill=None, body=float("nan")):
+        import torch
+        n = 1
+        for s in shape:
+            n *= s
+        self.guard, self.n = guard, n
+        self.buf = torch.empty(n + 2 * guard, dtype=dtype, device=device)
+        if fill is None:
+            g = torch.Generator(device=device).manual_seed(1234)
+            self.canary = torch.randn(2 * guard, generator=g, device=device).to(dtype)
+            self.buf[:guard] = self.canary[:guard]
+            self.buf[guard + n:] = self.canary[guard:]
+        else:
+            self.canary = None
+            self.buf.fill_(fill)
+        self.t = self.buf[guard:guard + n].view(shape)
+        self.t.fill_(body)
+
+    def canaries_intact(self):
+        import torch
+        if self.canary is None:
+            return True
+        got = torch.cat([self.buf[:self.guard], self.buf[self.guard + self.n:]])
+        return bool(torch.equal(got.view(torch.int16), self.canary.view(torch.int16)))
+
+
+def _guard_for(per_image):
+    return (per_image + 64 + 63) // 64 * 64  # one whole image (a store / load one image off) and then some
+
+
+def _conv_launch(L, ops, v, x, wp, op, out, out_relu, B, Hin, Win, Cin, N, cg, r1=None, r2=None):
+    vv = CONV_VARIANTS[v]
+    epi = {"chln": L.EPI_BF16_CHLN, "f16": L.EPI_F16}.get(vv.get("epi"), L.EPI_BF16)
+    ops.gemm(x, wp, conv=(B, Hin, Win, Cin), N=N, epi=epi, act=L.ACT_RELU if vv.get("act") == "relu" else L.ACT_NONE,
+             bias=op["b"] if vv.get("bias") else None,
+             gamma=op["lnw"] if vv.get("epi") == "chln" else None, aux=op["lnb"] if vv.get("epi") == "chln" else None,
+             resid1=r1 if vv.get("resid", 0) >= 1 else None, resid2=r2 if vv.get("resid", 0) >= 2 else None,
+             out_bf16=out, out_relu=out_relu, ldo=N, force_cg=cg, conv_stride=vv.get("stride", 1))
+
+
+def conv_tile_shape(B, H, W, pair):
+    import ctypes
+    sys.path.insert(0, ROOT)
+    from amodal_depth_anything_b200 import _lib as L
+    out = (ctypes.c_int64 * 4)()
+    L.check(L.load().ada_conv_tile_shape(B, H, W, pair, out))
+    return tuple(int(v) for v in out[:3])
+
+
+def chk_conv_geo(lw, lh, lb, pair, B, H, W, Cin, N, seed=0):
+    """One row of CONV_GEO_ROWS: the picker chooses the row's tile shape, and every epilogue variant passes
+    conv_geo_run with the row's pairing forced."""
+    res = conv_geo_run(B, H, W, Cin, N, pair, seed=seed)
+    res["shape"] = list(conv_tile_shape(B, H, W, pair))
+    res["ok"] = res["ok"] and res["shape"] == [lw, lh, lb]
+    return res
+
+
+def chk_conv_geo_bench(B, H, W, variants, ref_imgs):
+    """A batch-32 map of the ViT-L head (F = 256) with the launcher's own pairing, as the model runs it: more tiles than
+    SMs, so the persistent loop and both accumulator stages are exercised; fp64 on a few images, bit-equality with
+    one-image launches on all of them."""
+    res = conv_geo_run(B, H, W, 256, 256, 0, variants=variants, ref_imgs=ref_imgs, seed=8)  # even: odd stride-2 input
+    res["shapes"] = [list(conv_tile_shape(B, H, W, p)) for p in (1, 2)]
+    return res
+
+
+def conv_geo_run(B, H, W, Cin, N, cg, variants=tuple(CONV_VARIANTS), ref_imgs=None, seed=0):
+    """Every listed epilogue variant at one (B, H, W, Cin, N), force_cg=cg (0: the launcher's choice). Per variant: the
+    fp64 bound on the images `ref_imgs` (all if None), no unwritten pixel (outputs start as NaN), canaries around every
+    output intact, inputs and residuals inside NaN guards (conv padding must come from TMA's out-of-bounds zero fill), the
+    ReLU copy exact; every image bit-equal to a one-image launch (another tile shape); with cg=2 bit-equal to single-CTA
+    tiles."""
+    torch, L, ops = _imports()
+    dev = "cuda"
+    res = {"err_bound": 0.0, "variants": {}}
+    ok = True
+    t0 = time.time()
+    op = conv_geo_operands(B, H, W, Cin, N, seed, s2_odd=(seed % 2 == 0), device=dev, variants=variants)
+    imgs = list(range(B)) if ref_imgs is None else list(ref_imgs)
+    # fp64 reference on the host for the small rows, on the device for the large ones
+    ref_dev = dev if 18 * len(imgs) * H * W * Cin * N > 3e8 else "cpu"
+    ref_op = {k: (t[imgs] if k in ("x", "xs", "r1", "r2") else t).to(ref_dev) for k, t in op.items()}
+    wp = ops.pack_conv3x3(op["w"])
+    # inputs and residuals inside NaN guards, one image on either side
+    gin = {}
+    for k in ("x", "xs", "r1", "r2"):
+        if k in op:
+            t = op[k]
+            gin[k] = Guarded(tuple(t.shape), torch.bfloat16, dev, _guard_for(t[0].numel()), fill=float("nan"))
+            gin[k].t.copy_(t)
+    res_t = lambda k, i=None: None if k not in gin else gin[k].t if i is None else gin[k].t[i:i + 1]  # noqa: E731
+    for v in variants:
+        vv = CONV_VARIANTS[v]
+        s2 = vv.get("stride", 1) == 2
+        x = gin["xs" if s2 else "x"].t
+        Hin, Win = x.shape[1:3]
+        dt = torch.float16 if vv.get("epi") == "f16" else torch.bfloat16
+        guard = _guard_for(H * W * N)
+
+        def launch(xin, nb, r1, r2, c):
+            o = Guarded((nb, H, W, N), dt, dev, guard)
+            orl = Guarded((nb, H, W, N), dt, dev, guard) if vv.get("relu_copy") else None
+            _conv_launch(L, ops, v, xin, wp, op, o.t, orl.t if orl else None, nb, Hin, Win, Cin, N, c, r1, r2)
+            return o, orl
+
+        out, outr = launch(x, B, res_t("r1"), res_t("r2"), cg)
+        torch.cuda.synchronize()
+        ref, bound, relu_copy = conv_ref64(ref_op, v)
+        sel = torch.tensor(imgs, device=dev)
+        r = conv_verdict(out.t[sel], outr.t[sel] if outr else None, ref, bound, relu_copy)
+        if relu_copy:  # the ReLU copy of the images without an fp64 comparison too
+            r["relu_copy_exact"] = r["relu_copy_exact"] and bool(
+                torch.equal(outr.t.view(torch.int16), relu_copy_of(out.t).view(torch.int16)))
+        r["canaries_ok"] = out.canaries_intact() and (outr is None or outr.canaries_intact())
+        r["nan_all"] = int(torch.isnan(out.t.float()).sum().item())
+        # batch invariance: each image alone (B = 1 picks another tile shape) gives the same bits
+        same = True
+        for i in range(B):
+            o1, o1r = launch(x[i:i + 1], 1, res_t("r1", i), res_t("r2", i), 0)
+            same = same and torch.equal(o1.t.view(torch.int16), out.t[i:i + 1].view(torch.int16)) and o1.canaries_intact()
+            if o1r is not None:
+                same = same and torch.equal(o1r.t.view(torch.int16), outr.t[i:i + 1].view(torch.int16))
+        r["batch_invariant"] = bool(same)
+        if cg == 2:  # the same launch on single-CTA tiles
+            o2, o2r = launch(x, B, res_t("r1"), res_t("r2"), 1)
+            r["pair_invariant"] = bool(torch.equal(o2.t.view(torch.int16), out.t.view(torch.int16)) and
+                                       (o2r is None or torch.equal(o2r.t.view(torch.int16), outr.t.view(torch.int16))))
+        else:
+            r["pair_invariant"] = True
+        torch.cuda.synchronize()
+        r["ok"] = r["ok"] and r["canaries_ok"] and r["nan_all"] == 0 and r["batch_invariant"] and r["pair_invariant"]
+        res["variants"][v] = r
+        res["err_bound"] = max(res["err_bound"], r["err_bound"])
+        ok = ok and r["ok"]
+    res["inputs_untouched"] = all(bool(torch.equal(gin[k].t.view(torch.int16), op[k].view(torch.int16))) for k in gin)
+    res["ok"] = bool(ok and res["inputs_untouched"])
+    res["run_sec"] = round(time.time() - t0, 2)
+    return res
+
+
+# linear GEMM: the built (BN, CG) instantiations of each epilogue (ADA_GEMM_CASE in csrc/ada_api.cu)
+GEMM_TILES = {
+    "bf16": [(64, 1), (128, 1), (128, 2), (256, 1), (256, 2)],
+    "gelu": [(64, 1), (128, 1), (128, 2), (256, 1), (256, 2)],
+    "gamma": [(64, 1), (128, 1), (128, 2), (256, 1), (256, 2)],
+    "resid_f32": [(64, 1), (128, 1), (256, 1), (256, 2)],
+    "swiglu": [(128, 1), (256, 1), (256, 2)],
+    "f16": [(64, 1), (128, 1), (256, 1), (256, 2)],
+    "embed": [(64, 1), (128, 1), (256, 1), (256, 2)],
+}
+
+
+def chk_gemm_tiles(kind, M=1110, N=384, K=520, P=370):
+    """The tile of a linear GEMM (BN, CG; the small-launch cost model in launch_gemm picks among them) never changes a
+    bit: every built instantiation of the epilogue, and the launcher's own choice, give the same output. M is ragged
+    against 128 / 256 rows, N against 256 columns, K against 64. bf16 / gamma / fp32-residual / fp16 / embed outputs are
+    held to the fp64 bound; GELU and SwiGLU (tanh.approx) keep the tolerance of chk_gemm."""
+    torch, L, ops = _imports()
+    g = torch.Generator().manual_seed(31)
+    A = (torch.randn(M, K, generator=g) * 0.5).bfloat16()
+    Wt = (torch.randn(N, K, generator=g) * 0.05).bfloat16()
+    bias = torch.randn(N, generator=g) * 0.1
+    gam = 1.0 + 0.1 * torch.randn(N, generator=g)
+    x0 = torch.randn(M, N, generator=g) * 2
+    posb = torch.randn(P, N, generator=g)
+    acc = A.double() @ Wt.double().t()
+    S = A.double().abs() @ Wt.double().abs().t()
+    Ad, Wd = A.cuda(), Wt.cuda()
+    bd, gd, pd = bias.cuda(), gam.cuda(), posb.cuda()
+    rel, ref, tol = REL_BF16, acc + bias.double(), None
+    S = S + bias.double().abs()
+    if kind == "gamma":
+        ref, S = ref * gam.double(), S * gam.double().abs()
+    elif kind == "resid_f32":
+        ref, S, rel = ref * gam.double() + x0.double(), S * gam.double().abs() + x0.double().abs(), REL_F32
+    elif kind == "f16":
+        rel = REL_F16
+    elif kind == "embed":
+        ref = (acc.view(M // P, P, N) + posb.double()).view(M, N)
+        S, rel = (A.double().abs() @ Wt.double().abs().t()).view(M // P, P, N).add(posb.double().abs()).view(M, N), REL_F32
+    elif kind == "gelu":
+        ref, tol = torch.nn.functional.gelu(ref), (2e-2, 1e-2)
+    elif kind == "swiglu":
+        ref, tol = torch.nn.functional.silu(ref[:, :N // 2]) * ref[:, N // 2:], (2e-2, 1e-2)
+    idx = torch.arange(N)
+    src = torch.where(idx % 64 < 32, idx // 64 * 32 + idx % 64, N // 2 + idx // 64 * 32 + idx % 64 - 32)  # as ada_finalize
+
+    def run(bn, cg):
+        if kind == "resid_f32":
+            out = x0.clone().cuda()
+            ops.gemm(Ad, Wd, epi=L.EPI_RESID_F32, bias=bd, gamma=gd, out_f32=out, ldo=N, force_bn=bn, force_cg=cg)
+        elif kind == "embed":
+            out = torch.full((M // P, P + 1, N), 7.0, device="cuda")
+            ops.gemm(Ad, Wd, epi=L.EPI_EMBED, aux=pd, out_f32=out, ldo=N, P=P, force_bn=bn, force_cg=cg)
+        elif kind == "swiglu":
+            out = torch.full((M, N // 2), float("nan"), dtype=torch.bfloat16, device="cuda")
+            ops.gemm(Ad, Wd[src.cuda()].contiguous(), epi=L.EPI_SWIGLU, bias=bd[src.cuda()].contiguous(), out_bf16=out,
+                     ldo=N // 2, force_bn=bn, force_cg=cg)
+        else:
+            dt = torch.float16 if kind == "f16" else torch.bfloat16
+            out = torch.full((M, N), float("nan"), dtype=dt, device="cuda")
+            ops.gemm(Ad, Wd, epi=L.EPI_F16 if kind == "f16" else L.EPI_BF16, act=L.ACT_GELU if kind == "gelu" else L.ACT_NONE,
+                     bias=bd, gamma=gd if kind == "gamma" else None, out_bf16=out, ldo=N, force_bn=bn, force_cg=cg)
+        torch.cuda.synchronize()
+        return out
+
+    first = run(*GEMM_TILES[kind][0])
+    same = {}
+    for bn, cg in GEMM_TILES[kind][1:] + [(0, 0)]:
+        o = run(bn, cg)
+        same[f"{bn}x{cg}" if bn else "auto"] = bool(torch.equal(o.view(torch.int32 if o.dtype == torch.float32 else torch.int16),
+                                                               first.view(torch.int32 if o.dtype == torch.float32 else torch.int16)))
+    got = first.cpu()
+    r = {"same_bits": same}
+    if kind == "embed":
+        r["cls_untouched"] = bool((got[:, 0] == 7.0).all().item())
+        got = got[:, 1:].reshape(M, N)
+    if tol is None:
+        r["err_bound"] = err_over_bound(got, ref, REL_ACC * S + rel * ref.abs())
+        r["ok"] = r["err_bound"] <= 1.0
+    else:
+        c = _cmp(kind, got, ref.float(), *tol)
+        r.update(max_abs=c["max_abs"], bad=c["bad"])
+        r["ok"] = c["ok"]
+    r["nan"] = int(torch.isnan(got.float()).sum().item())
+    r["ok"] = bool(r["ok"] and r["nan"] == 0 and all(same.values()) and r.get("cls_untouched", True))
+    return r
+
+
 CHECKS = {
     "gemm_resid_f32": lambda: chk_gemm_resid_f32(1370 * 3, 1024, 1024),
     "gemm_resid_f32_cg2": lambda: chk_gemm_resid_f32(1370 * 3, 1024, 4096, cg=2),
@@ -470,6 +870,13 @@ CHECKS = {
     "conv_s2_37": lambda: chk_conv_s2(2, 37, 37, 128, 192),
     "conv_s2_74x50": lambda: chk_conv_s2(1, 74, 50, 64, 64),
     "conv_s2_1024": lambda: chk_conv_s2(2, 37, 37, 1024, 1024),
+    # every pixel-tile shape x every conv epilogue against fp64 (seeded by row; odd seeds give the stride-2 input an even size)
+    **{f"conv_geo_{r[0]}{r[1]}{r[2]}_{r[3]}": (lambda r=r, i=i: chk_conv_geo(*r, seed=i)) for i, r in enumerate(CONV_GEO_ROWS)},
+    # batch-32 maps of the ViT-L head: layer_rn, RCU1 conv2, plain conv; resize_layers[3] 37 -> 19
+    **{f"conv_geo_bench_{h}": (lambda h=h: chk_conv_geo_bench(32, h, h, ("a_bias", "b_relu_copy", "d_resid2_relu_copy"),
+                                                              (0, 16, 31))) for h in (148, 74, 37, 19)},
+    "conv_geo_bench_s2_37": lambda: chk_conv_geo_bench(32, 19, 19, ("h_s2_bias",), (0, 16, 31)),
+    **{f"gemm_tiles_{k}": (lambda k=k: chk_gemm_tiles(k)) for k in GEMM_TILES},
 }
 
 
