@@ -556,7 +556,7 @@ static void launch_attention(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B
   a.scale_log2e = 0.125f * 1.4426950408889634f;
   dim3 grid((N + kAttQ - 1) / kAttQ, heads, B);
   ProfScope prof(PC_ATTENTION, 4.0 * B * heads * static_cast<double>(N) * N * 64.0, 8.0 * B * static_cast<double>(N) * D, st);
-  // Two kernels that agree bit for bit (tools/gpu_check.py attention_impls_agree_*). attention.cuh (one 128-query tile per
+  // Two kernels that agree bit for bit (tools/gpu_check.py attention_geo_*). attention.cuh (one 128-query tile per
   // CTA, two CTAs per SM, a score row shared by two threads) is the product path. attention2.cuh (persistent CTAs, 256
   // queries per work unit, one thread per score row, three issuing warps) is selectable with ADA_ATT_IMPL=1 / impl = 1 of
   // ada_op_attention: round-2 measurements (profiles/README.md) put it 3-6 % ahead stand-alone and in the model when ALL

@@ -109,7 +109,7 @@ __device__ __forceinline__ FaUnit fa_unit(int idx, const FaArgs& a) {
 // softmax warps per scheduler a warp's phases (wait, tcgen05.ld, maximum, exponentials, tcgen05.st) are simply serialised;
 // four warps per scheduler let one warp's exponentials (MUFU) overlap the others' fixed-latency phases.
 // Measured (B200, 32 x 1370 x 16 heads): 0.393 ms, against 0.360 ms for one thread per row and 0.350 ms for attention.cuh;
-// bit-identical to both (tools/gpu_check.py attention_impls_agree_*). The pair exchange through shared memory and the 104
+// bit-identical to both (tools/gpu_check.py attention_geo_*). The pair exchange through shared memory and the 104
 // register cap (a few spills in the exponential loop) cost more than the extra warps hide; kept as impl = 2 for the record.
 template <int EMU, bool STAGGER, int WAITP, bool SPLIT = false>
 __global__ void __launch_bounds__(SPLIT ? kFaThreadsSplit : kFaThreads, 1)

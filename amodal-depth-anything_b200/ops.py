@@ -56,31 +56,42 @@ def gemm(A, Wt, *, epi=L.EPI_BF16, act=L.ACT_NONE, bias=None, gamma=None, resid_
     _call(A, lib.ada_op_gemm, ctypes.byref(d))
 
 
-def layernorm(x, w, b, eps=1e-6, n_tok=0, drop_cls=False, delta=None, write_x=False, delta2=None, tap_w=None, tap_b=None):
-    """tap_w / tap_b: also return a second affine of the same normalised rows as the cls-less patch map (needs n_tok)."""
+def layernorm(x, w, b, eps=1e-6, n_tok=0, drop_cls=False, delta=None, write_x=False, delta2=None, tap_w=None, tap_b=None,
+              out=None, out2=None):
+    """tap_w / tap_b: also return a second affine of the same normalised rows as the cls-less patch map (needs n_tok).
+    out / out2: bf16 outputs to store into (allocated when None)."""
     rows, D = x.shape
-    if drop_cls:
-        out = torch.empty((rows // n_tok) * (n_tok - 1), D, dtype=torch.bfloat16, device=x.device)
+    out_rows = (rows // n_tok) * (n_tok - 1) if drop_cls else rows
+    if out is None:
+        out = torch.empty(out_rows, D, dtype=torch.bfloat16, device=x.device)
+    assert out.shape == (out_rows, D) and out.dtype == torch.bfloat16 and out.is_contiguous()
+    if tap_w is None:
+        out2 = None
     else:
-        out = torch.empty(rows, D, dtype=torch.bfloat16, device=x.device)
-    out2 = None
-    if tap_w is not None:
-        out2 = torch.empty((rows // n_tok) * (n_tok - 1), D, dtype=torch.bfloat16, device=x.device)
+        if out2 is None:
+            out2 = torch.empty((rows // n_tok) * (n_tok - 1), D, dtype=torch.bfloat16, device=x.device)
+        assert out2.shape == ((rows // n_tok) * (n_tok - 1), D) and out2.dtype == torch.bfloat16 and out2.is_contiguous()
     _call(x, L.load().ada_op_layernorm, _p(x), _p(delta), _p(delta2), _p(w), _p(b), _p(out), rows, D, eps, n_tok, int(drop_cls),
           int(write_x), _p(tap_w), _p(tap_b), _p(out2))
     return out if out2 is None else (out, out2)
 
 
-def attention(qkv, B, N, heads, impl=-1):
-    """impl: -1 = the kernel the model would use at this shape, 0 / 1 / 2 = force attention.cuh / attention2.cuh (one thread per row) / attention2.cuh (two threads per row)."""
-    out = torch.empty(B * N, heads * 64, dtype=torch.bfloat16, device=qkv.device)
+def attention(qkv, B, N, heads, impl=-1, out=None):
+    """impl: -1 = the kernel the model would use at this shape, 0 / 1 / 2 = force attention.cuh / attention2.cuh (one thread per row) / attention2.cuh (two threads per row).
+    out: bf16 [B * N, heads * 64] to store into (allocated when None)."""
+    if out is None:
+        out = torch.empty(B * N, heads * 64, dtype=torch.bfloat16, device=qkv.device)
+    assert out.shape == (B * N, heads * 64) and out.dtype == torch.bfloat16 and out.is_contiguous()
     _call(qkv, L.load().ada_op_attention, _p(qkv), _p(out), B, N, heads, impl)
     return out
 
 
-def channel_ln_relu(x_nhwc, w, b, eps=1e-6):
+def channel_ln_relu(x_nhwc, w, b, eps=1e-6, out=None):
+    """out: bf16 tensor of x_nhwc's shape to store into (allocated when None; x_nhwc itself is allowed)."""
     C = x_nhwc.shape[-1]
-    out = torch.empty_like(x_nhwc)
+    if out is None:
+        out = torch.empty_like(x_nhwc)
+    assert out.shape == x_nhwc.shape and out.dtype == torch.bfloat16 and out.is_contiguous()
     _call(x_nhwc, L.load().ada_op_channel_ln_relu, _p(x_nhwc), _p(w), _p(b), _p(out), x_nhwc.numel() // C, C, eps)
     return out
 

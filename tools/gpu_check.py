@@ -155,134 +155,6 @@ def chk_convT(ks, Cin=96, Cout=96, B=2, H=37, W=37, pix=False):
     return _cmp("convT", out.permute(0, 3, 1, 2), ref, 3e-2, 1e-2)
 
 
-def chk_attention(B, N, heads, grow=False, impl=-1):
-    torch, L, ops = _imports()
-    g = torch.Generator(device="cuda").manual_seed(5)
-    D = heads * 64
-    qkv = torch.randn(B, N, 3, heads, 64, generator=g, device="cuda") * 1.5
-    if grow:  # key norms grow along the sequence -> row maxima jump by > 2^8 between KV tiles (exercises the O rescale)
-        ramp = 1.0 + 7.0 * (torch.arange(N, device="cuda") // 128).float() / max((N - 1) // 128, 1)
-        qkv[:, :, 1] *= ramp.view(1, N, 1, 1)
-    qkv = qkv.bfloat16()
-    out = ops.attention(qkv, B, N, heads, impl)
-    torch.cuda.synchronize()
-    q, k, v = [t.float().permute(0, 2, 1, 3) for t in qkv.unbind(2)]  # [B,h,N,64]
-    att = torch.softmax((q * 0.125) @ k.transpose(-1, -2), dim=-1)
-    ref = (att @ v).permute(0, 2, 1, 3).reshape(B * N, D)
-    return _cmp("attention", out, ref, 2e-2, 2e-2)
-
-
-def chk_attention_impls_agree(B, N, heads, grow=False):
-    """The two attention kernels are selected by grid size; an image must not change with the batch it is processed in, so
-    they have to agree bit for bit (same exponential evaluation per column, same summation order of the row sums)."""
-    torch, L, ops = _imports()
-    g = torch.Generator(device="cuda").manual_seed(15)
-    qkv = torch.randn(B, N, 3, heads, 64, generator=g, device="cuda") * 1.5
-    if grow:
-        ramp = 1.0 + 7.0 * (torch.arange(N, device="cuda") // 128).float() / max((N - 1) // 128, 1)
-        qkv[:, :, 1] *= ramp.view(1, N, 1, 1)
-    qkv = qkv.bfloat16()
-    a = ops.attention(qkv, B, N, heads, 0)
-    worst, n_diff, ok = 0.0, 0, True
-    for impl in (1, 2):
-        b = ops.attention(qkv, B, N, heads, impl)
-        torch.cuda.synchronize()
-        diff = (a.float() - b.float()).abs()
-        ok = ok and bool(torch.equal(a, b))
-        worst = max(worst, diff.max().item())
-        n_diff += int((diff > 0).sum().item())
-    return {"ok": ok, "max_abs": worst, "n_diff": n_diff, "n": a.numel()}
-
-
-def chk_layernorm(D, drop):
-    torch, L, ops = _imports()
-    g = torch.Generator(device="cuda").manual_seed(6)
-    B, n_tok = 3, 50
-    x = torch.randn(B * n_tok, D, generator=g, device="cuda") * 2 + 0.5
-    w = torch.randn(D, generator=g, device="cuda")
-    b = torch.randn(D, generator=g, device="cuda")
-    out = ops.layernorm(x, w, b, 1e-6, n_tok, drop)
-    torch.cuda.synchronize()
-    ref = torch.nn.functional.layer_norm(x, (D,), w, b, 1e-6)
-    if drop:
-        ref = ref.view(B, n_tok, D)[:, 1:].reshape(-1, D)
-    return _cmp("ln", out, ref, 2e-2, 1e-2)
-
-
-def chk_layernorm_delta():
-    torch, L, ops = _imports()
-    g = torch.Generator(device="cuda").manual_seed(16)
-    rows, D = 300, 1024
-    x = torch.randn(rows, D, generator=g, device="cuda") * 2
-    d = torch.randn(rows, D, generator=g, device="cuda").bfloat16()
-    w = torch.randn(D, generator=g, device="cuda")
-    b = torch.randn(D, generator=g, device="cuda")
-    x1 = x.clone()
-    out = ops.layernorm(x1, w, b, 1e-6, 1, False, delta=d, write_x=True)
-    x2 = x.clone()
-    out2 = ops.layernorm(x2, w, b, 1e-6, 1, False, delta=d, write_x=False)
-    torch.cuda.synchronize()
-    xs = x + d.float()
-    ref = torch.nn.functional.layer_norm(xs, (D,), w, b, 1e-6)
-    r = _cmp("ln", out, ref, 2e-2, 1e-2)
-    r["x_written"] = bool(torch.equal(x1, xs))
-    r["x_untouched"] = bool(torch.equal(x2, x))
-    r["ok"] = r["ok"] and r["x_written"] and r["x_untouched"] and bool(torch.equal(out, out2))
-    # two pending branches: (x + d) + d2, the order the encoder relies on (norm2 sees x + d, the next norm1 adds d2)
-    d2 = torch.randn(rows, D, generator=g, device="cuda").bfloat16()
-    x3 = x.clone()
-    out3 = ops.layernorm(x3, w, b, 1e-6, 1, False, delta=d, write_x=True, delta2=d2)
-    torch.cuda.synchronize()
-    xs2 = (x + d.float()) + d2.float()
-    r2 = _cmp("ln2", out3, torch.nn.functional.layer_norm(xs2, (D,), w, b, 1e-6), 2e-2, 1e-2)
-    r["x_written_2"] = bool(torch.equal(x3, xs2))
-    r["ok"] = r["ok"] and r2["ok"] and r["x_written_2"]
-    return r
-
-
-def chk_layernorm_tap():
-    """norm1 of the next block and the tap of the previous one in one pass: same statistics, two affines, the second written
-    without the cls rows (dinov2.py:337-340)."""
-    torch, L, ops = _imports()
-    g = torch.Generator(device="cuda").manual_seed(26)
-    B, n_tok, D = 3, 50, 1024
-    x = torch.randn(B * n_tok, D, generator=g, device="cuda") * 2 + 0.3
-    d1 = torch.randn(B * n_tok, D, generator=g, device="cuda").bfloat16()
-    d2 = torch.randn(B * n_tok, D, generator=g, device="cuda").bfloat16()
-    w, b, w2, b2 = (torch.randn(D, generator=g, device="cuda") for _ in range(4))
-    x1 = x.clone()
-    out, tap = ops.layernorm(x1, w, b, 1e-6, n_tok, False, delta=d1, write_x=True, delta2=d2, tap_w=w2, tap_b=b2)
-    torch.cuda.synchronize()
-    xs = (x + d1.float()) + d2.float()
-    r = _cmp("ln", out, torch.nn.functional.layer_norm(xs, (D,), w, b, 1e-6), 2e-2, 1e-2)
-    ref2 = torch.nn.functional.layer_norm(xs, (D,), w2, b2, 1e-6).view(B, n_tok, D)[:, 1:].reshape(-1, D)
-    r2 = _cmp("tap", tap, ref2, 2e-2, 1e-2)
-    # the separate tap pass (what the last block still uses) must give the same bits
-    x2 = x.clone()
-    tap_alone = ops.layernorm(x2, w2, b2, 1e-6, n_tok, True, delta=d1, write_x=False, delta2=d2)
-    torch.cuda.synchronize()
-    r["tap_ok"] = r2["ok"]
-    r["tap_same_bits_as_separate_pass"] = bool(torch.equal(tap, tap_alone))
-    r["x_written"] = bool(torch.equal(x1, xs))
-    r["ok"] = r["ok"] and r2["ok"] and r["tap_same_bits_as_separate_pass"] and r["x_written"]
-    return r
-
-
-def chk_channel_ln(C):
-    torch, L, ops = _imports()
-    g = torch.Generator(device="cuda").manual_seed(7)
-    x = (torch.randn(2, 9, 11, C, generator=g, device="cuda") * 2 + 0.3).bfloat16()
-    w = torch.randn(C, generator=g, device="cuda")
-    b = torch.randn(C, generator=g, device="cuda")
-    out = ops.channel_ln_relu(x, w, b)
-    torch.cuda.synchronize()
-    xf = x.float()
-    u = xf.mean(-1, keepdim=True)
-    s = (xf - u).pow(2).mean(-1, keepdim=True)
-    ref = torch.relu((xf - u) / torch.sqrt(s + 1e-6) * w + b)
-    return _cmp("cln", out, ref, 2e-2, 1e-2)
-
-
 def chk_upsample(Hi, Ho, C=64):
     torch, L, ops = _imports()
     g = torch.Generator(device="cuda").manual_seed(8)
@@ -792,6 +664,409 @@ def chk_gemm_tiles(kind, M=1110, N=384, K=520, P=370):
     return r
 
 
+# ---- attention: every ragged sequence length and head count the model can launch, against an fp64 reference
+#
+# Error model, per query row i of one (image, head), with a_ij = softmax_j(s_ij / 8), ref_i = sum_j a_ij v_j and
+# R_i = sum_j a_ij |v_j| (fp64 from the bf16 inputs):
+#   2^-8 |ref_i|                     the bf16 output rounding;
+#   2^-8 R_i                         P is stored as bf16 (relative error <= 2^-8 per key) while the row sum adds the
+#                                    unrounded fp32 p, so the output is sum_j a_ij (1 + d_j) v_j with |d_j| <= 2^-8;
+#   2 EXP_EPS (R_i + |ref_i|)        the exponential (FMA-pipe polynomial or MUFU ex2) moves every weight by a relative
+#                                    error <= EXP_EPS; normalising by the row sum of the same p doubles it, and a common
+#                                    weight change cancels against ref_i, hence |v_j - ref_i| <= |v_j| + |ref_i|;
+#   N 2^-24 (R_i + |ref_i|)          the fp32 row sum and the fp32 P V accumulation over N keys;
+#   2 sum_j a_ij e_ij (|v_j| + |ref_i|), e_ij = 2^-16 (|q_i| . |k_j|) / 8
+#                                    the fp32 score accumulation (64 exact bf16 products) moves p_j by a relative e_ij;
+#                                    the factor 2 covers exp(e) - 1 <= 2 e for e <= 1.
+# The fp32 rounding of x = s c - m c (c = 0.125 log2 e) adds at most 2^-23 |x| ln 2 per weight; weighted by a_ij that
+# is below 2^-18 for any row, inside the slack EXP_EPS keeps over the measured polynomial error.
+# EXP_EPS: the FMA-pipe exp2 polynomial (ptx.cuh exp2_fma2) has a measured maximum relative error of 7.5e-5 (2^-13.7) over
+# [-125, 8]; MUFU ex2.approx is good to ~2^-22. tests/test_encoder_check_cpu.py re-measures it and the P-rounding term.
+EXP_EPS = 2.0 ** -13
+ATT_MODES = ("rand", "neg", "peak_last", "peak_first", "grow", "grow8", "wide")
+_ATT_BASE = ("rand", "neg", "peak_last", "peak_first")
+_ATT_GROW = _ATT_BASE + ("grow", "grow8")
+
+# (B, N, heads, modes, ref_pairs). Any N is a real launch (a 14 x 14 (N - 1) image has N tokens), so the table walks the
+# residues N mod 128 at the edges of both kernels: N < 128 (a single ragged tile; 64 = the boundary of the two 64-column
+# halves of a score row in attention.cuh), r = 1 (the second-half thread of every row has no key), 32 / 33 and 64 / 65
+# (attention2.cuh skips 32-key chunks entirely past N), 127. N = 129 / 257 / 1409 put a single row in a query tile of
+# attention2.cuh (the second tile of a full unit / a short unit). Heads 6 / 12 / 16 / 24 = ViT-S / B / L / G.
+# ref_pairs: (image, head) pairs held to the fp64 bound on the largest rows; bit-equality with the one-image launches
+# and across the kernels covers the others.
+ATT_ROWS = [
+    (3, 2, 6, _ATT_BASE, None),
+    (2, 17, 24, _ATT_BASE, None),           # ViT-G at 56 x 56
+    (2, 33, 12, _ATT_BASE, None),
+    (2, 64, 6, _ATT_BASE + ("wide",), None),  # the 126 x 98 golden
+    (2, 65, 16, _ATT_BASE, None),
+    (1, 128, 1, _ATT_BASE, None),
+    (2, 128, 12, _ATT_BASE, None),
+    (10, 128, 16, _ATT_BASE, None),         # several work units per persistent CTA
+    (2, 129, 6, _ATT_BASE, None),
+    (1, 160, 24, _ATT_BASE, None),
+    (2, 191, 16, _ATT_BASE, None),
+    (1, 200, 2, _ATT_BASE, None),
+    (1, 257, 12, _ATT_GROW, None),
+    (1, 289, 6, _ATT_GROW, None),
+    (8, 300, 16, _ATT_GROW, None),          # full and short units interleaved
+    (2, 320, 16, _ATT_GROW + ("wide",), None),
+    (1, 383, 24, _ATT_GROW, None),
+    (2, 700, 16, _ATT_GROW, None),
+    (3, 700, 16, _ATT_GROW, None),
+    (1, 1370, 2, _ATT_GROW, None),
+    (2, 1370, 6, _ATT_GROW + ("wide",), None),  # ViT-S at 518 x 518
+    (3, 1370, 16, _ATT_GROW, None),
+    (4, 1370, 16, _ATT_GROW, None),
+    (1, 1409, 12, _ATT_GROW, None),
+    (1, 1814, 6, _ATT_GROW + ("wide",), None),  # 518 x 686
+    (1, 5477, 2, _ATT_GROW, None),
+    (1, 5477, 4, _ATT_GROW, ((0, 0), (0, 3))),
+    (1, 5477, 6, _ATT_GROW, ((0, 0), (0, 5))),
+    (32, 1370, 6, _ATT_GROW, ((0, 0), (13, 2), (31, 5))),
+    (32, 1370, 16, _ATT_GROW, ((0, 0), (16, 7), (31, 15))),  # the benchmark's ViT-L launch
+]
+
+
+def att_operands(B, N, heads, mode, seed, device="cpu"):
+    """qkv [B, N, 3, heads, 64] bf16 of one input mode (v is 1.5 N(0, 1) throughout):
+    rand        q, k ~ 1.5 N(0, 1);
+    neg         q >= 0, k <= 0 elementwise: every real score is clearly negative, so a key past N that escapes the mask
+                (score 0, v 0) takes most of the weight;
+    peak_last / peak_first   one key (N - 1, inside the ragged tile / 0) leads every row by ~24 logits (q[0] = 4,
+                k[0] = 48 there and 0 elsewhere): masking a real key, or mixing up keys, changes the output completely;
+    grow        key norms ramp 1 -> 8 over the KV tiles: row maxima jump by more than 2^8 between tiles (O rescale);
+    grow8       the keys of KV tile t carry k[0] = 10.375 t with q[0] = 4: every tile's maximum is ~7.5 (log2 units)
+                above the previous one, just under the 2^8 rescale threshold, so p reaches ~2^7.5 without a rescale
+                on every other tile;
+    wide        q, k ~ 7.5 N(0, 1): scores span about +-200 logits, most p underflow, and the score error dominates."""
+    import torch
+    g = torch.Generator(device=device).manual_seed(seed)
+    qkv = torch.randn(B, N, 3, heads, 64, generator=g, device=device) * 1.5
+    q, k = qkv[:, :, 0], qkv[:, :, 1]
+    if mode == "neg":
+        q.abs_()
+        k.abs_().neg_()
+    elif mode in ("peak_last", "peak_first"):
+        q[..., 1:] *= 0.5
+        q[..., 0] = 4.0
+        k[..., 0] = 0.0
+        k[:, N - 1 if mode == "peak_last" else 0, :, 0] = 48.0
+    elif mode == "grow":
+        ramp = 1.0 + 7.0 * (torch.arange(N, device=device) // 128).float() / max((N - 1) // 128, 1)
+        k *= ramp.view(1, N, 1, 1)
+    elif mode == "grow8":
+        q[..., 1:] *= 0.02
+        q[..., 0] = 4.0
+        k[..., 0] = 10.375 * (torch.arange(N, device=device) // 128).float().view(1, N, 1)
+    elif mode == "wide":
+        q *= 5.0
+        k *= 5.0
+    else:
+        assert mode == "rand", mode
+    return qkv.bfloat16()
+
+
+def att_ref64(qkv, pairs=None, device="cpu", chunk=1024):
+    """fp64 reference and per-element bound (error model above) of attention on qkv [B, N, 3, heads, 64] for the
+    (image, head) pairs `pairs` (all if None): (ref, bound), each [len(pairs), N, 64] fp64 on `device`."""
+    import torch
+    B, N, _, H, _ = qkv.shape
+    pairs = [(b, h) for b in range(B) for h in range(H)] if pairs is None else list(pairs)
+    refs, bounds = [], []
+    for b, h in pairs:
+        q, k, v = (qkv[b, :, i, h].to(device).double() for i in range(3))
+        ka, va = k.abs(), v.abs()
+        ref = torch.empty(N, 64, dtype=torch.float64, device=device)
+        bound = torch.empty_like(ref)
+        for i0 in range(0, N, chunk):
+            qc = q[i0:i0 + chunk]
+            a = torch.softmax((qc @ k.t()) * 0.125, dim=-1)
+            r = a @ v
+            R = a @ va
+            ae = a * (qc.abs() @ ka.t()) * (REL_ACC / 8)
+            ra = r.abs()
+            ref[i0:i0 + chunk] = r
+            bound[i0:i0 + chunk] = (REL_BF16 * (ra + R) + (2 * EXP_EPS + N * 2.0 ** -24) * (R + ra) +
+                                    2 * (ae @ va + ae.sum(-1, keepdim=True) * ra))
+        refs.append(ref)
+        bounds.append(bound)
+    return torch.stack(refs), torch.stack(bounds)
+
+
+def att_select(out, B, N, heads, pairs):
+    """The (image, head) pairs of an attention output [B * N, heads * 64] as [len(pairs), N, 64]."""
+    import torch
+    o = out.view(B, N, heads, 64)
+    return torch.stack([o[b, :, h] for b, h in pairs])
+
+
+def att_verdict(got, ref, bound):
+    """got / ref / bound [pairs, N, 64]: within the bound everywhere, no NaN."""
+    import torch
+    r = {"err_bound": err_over_bound(got, ref, bound), "nan": int(torch.isnan(got.float()).sum().item())}
+    r["ok"] = r["err_bound"] <= 1.0 and r["nan"] == 0
+    return r
+
+
+def chk_attention_geo(B, N, heads, modes, ref_pairs=None, seed=0, impls=(0, 1, 2, -1)):
+    """One row of ATT_ROWS, every listed input mode: qkv inside a NaN-filled buffer with one image of guard on either side
+    (keys past N must come from the tensor map's zero fill), every output in a canary-guarded buffer that starts as NaN
+    (unwritten rows, stores of the ragged query tile past N). Per mode: the listed impls (0 / 1 / 2, -1 = the default)
+    bit-identical, every image launched alone (with the last listed impl) bit-equal to the same image in the batch, qkv
+    unchanged, no NaN, canaries intact, and err_over_bound <= 1 on every (image, head) or on ref_pairs."""
+    torch, L, ops = _imports()
+    dev = "cuda"
+    D = heads * 64
+    pairs = [(b, h) for b in range(B) for h in range(heads)] if ref_pairs is None else list(ref_pairs)
+    ref_dev = dev if 4 * len(pairs) * N * N * 64 > 2e9 else "cpu"
+    res = {"err_bound": 0.0, "modes": {}}
+    ok = True
+    t0 = time.time()
+    i16 = torch.int16
+    for mi, mode in enumerate(modes):
+        qkv = att_operands(B, N, heads, mode, seed * 16 + mi, device=dev)
+        gq = Guarded(tuple(qkv.shape), torch.bfloat16, dev, _guard_for(N * 3 * D), fill=float("nan"))
+        gq.t.copy_(qkv)
+
+        def launch(x, nb, impl):
+            o = Guarded((nb * N, D), torch.bfloat16, dev, _guard_for(N * D))
+            ops.attention(x, nb, N, heads, impl, out=o.t)
+            return o
+
+        outs = {impl: launch(gq.t, B, impl) for impl in impls}
+        torch.cuda.synchronize()
+        base = outs[impls[0]].t
+        r = att_verdict(att_select(base, B, N, heads, pairs).to(ref_dev), *att_ref64(qkv, pairs, ref_dev))
+        r["impls_same_bits"] = all(bool(torch.equal(outs[i].t.view(i16), base.view(i16))) for i in impls[1:])
+        r["canaries_ok"] = all(o.canaries_intact() for o in outs.values())
+        r["nan_all"] = sum(int(torch.isnan(o.t.float()).sum().item()) for o in outs.values())
+        same = True
+        if B > 1:  # each image alone: another grid, another unit list
+            for i in range(B):
+                o1 = launch(gq.t[i:i + 1], 1, impls[-1])
+                same = same and bool(torch.equal(o1.t.view(i16), base[i * N:(i + 1) * N].view(i16))) and o1.canaries_intact()
+        r["batch_invariant"] = same
+        r["qkv_untouched"] = bool(torch.equal(gq.t.view(i16), qkv.view(i16)))
+        torch.cuda.synchronize()
+        r["ok"] = bool(r["ok"] and r["impls_same_bits"] and r["canaries_ok"] and r["nan_all"] == 0 and r["batch_invariant"]
+                       and r["qkv_untouched"])
+        res["modes"][mode] = r
+        res["err_bound"] = max(res["err_bound"], r["err_bound"])
+        ok = ok and r["ok"]
+        del qkv, gq, outs
+    res["ok"] = bool(ok)
+    res["run_sec"] = round(time.time() - t0, 2)
+    return res
+
+
+# ---- token LayerNorm and channel LayerNorm: one fp64 reference and bound for both kernels
+#
+# Error model: the kernels compute fp32 two-pass statistics (mean, then the mean of squared deviations) of the row they
+# normalise. The mean is off by well under 2^-16 mean|x| (D <= 1536 terms, per-lane partial sums and a warp tree), which
+# moves every output by |w| rstd times that; the variance (and hence rstd) is good to a few 2^-24, far under 2^-16
+# relative, which moves an output by 2^-16 |w| rstd |x - mean|. The affine (x - mean) * rstd * w + b in fp32 adds
+# 2^-22 |b| where the two terms cancel, and the bf16 store 2^-8 |ref|. ReLU (channel LN) is 1-Lipschitz.
+LN_EPS = 1e-6
+LN_ROW_KINDS = ("normal", "offset", "massive", "near_const", "const")
+# Common offset of the "offset" rows (sigma 1): a one-pass variance E[x^2] - E[x]^2 in fp32 loses all of its digits there
+# (tests/test_encoder_check_cpu.py shows it fails the bound); the two-pass statistics pass with a wide margin.
+LN_OFFSET = 3000.0
+
+
+def ln_operands(rows, D, seed, device="cpu", deltas=False):
+    """x [rows, D] fp32 mixing the row kinds (row r is LN_ROW_KINDS[r % 5]): N(0, s) with s in [0.5, 4]; LN_OFFSET +
+    N(0, 1); N(0, 1) with four +-500 "massive activation" columns; c + 1e-3 N(0, 1) (eps is as large as the variance);
+    exactly constant. w, b, w2, b2: fp32 affines. deltas: also d, d2 (bf16 [rows, D], the pending residual branches)
+    that keep each row's kind: N(0, 1) on the first three kinds, 1e-3 N(0, 1) on the near-constant rows, one constant per
+    row on the constant rows."""
+    import torch
+    g = torch.Generator(device=device).manual_seed(seed)
+    rnd = lambda *s: torch.randn(*s, generator=g, device=device)  # noqa: E731
+    kind = torch.arange(rows, device=device) % len(LN_ROW_KINDS)
+    z = rnd(rows, D)
+    c = rnd(rows, 1)
+    s = 0.5 + 3.5 * torch.rand(rows, 1, generator=g, device=device)
+    massive = z.clone()
+    cols = torch.randint(0, D, (rows, 4), generator=g, device=device)
+    massive.scatter_(1, cols, 500.0 * torch.sign(rnd(rows, 4)))
+    cases = [z * s + 0.3 * c, LN_OFFSET + z, massive, c + 1e-3 * z, c.expand(rows, D)]
+    x = torch.zeros(rows, D, device=device)
+    for i, t in enumerate(cases):
+        x = torch.where((kind == i).view(rows, 1), t, x)
+    op = {"x": x.contiguous(), "kind": kind}
+    for nm in ("w", "b", "w2", "b2"):
+        op[nm] = rnd(D)
+    if deltas:
+        for nm in ("d", "d2"):
+            zd, cd = rnd(rows, D), rnd(rows, 1)
+            t = torch.where((kind == 3).view(rows, 1), 1e-3 * zd, zd)
+            op[nm] = torch.where((kind == 4).view(rows, 1), cd.expand(rows, D), t).bfloat16()
+    return op
+
+
+def ln_ref64(x, w, b, relu=False, eps=LN_EPS):
+    """fp64 LayerNorm (x - mean) * rstd * w + b over the last dim (ReLU'd for the channel LN) of fp32 / bf16 rows x, and
+    the per-element bound of the error model above: (ref, bound), fp64 on x's device."""
+    import torch
+    xd = x.double()
+    mean = xd.mean(-1, keepdim=True)
+    xc = xd - mean
+    rstd = 1.0 / torch.sqrt(xc.pow(2).mean(-1, keepdim=True) + eps)
+    wd, bd = w.double().to(x.device), b.double().to(x.device)
+    ref = xc * rstd * wd + bd
+    if relu:
+        ref = torch.relu(ref)
+    bound = REL_BF16 * ref.abs() + REL_ACC * wd.abs() * rstd * (xc.abs() + xd.abs().mean(-1, keepdim=True)) + REL_F32 * bd.abs()
+    return ref, bound
+
+
+def ln_verdict(got, ref, bound):
+    import torch
+    r = {"err_bound": err_over_bound(got, ref, bound), "nan": int(torch.isnan(got.float()).sum().item())}
+    r["ok"] = r["err_bound"] <= 1.0 and r["nan"] == 0
+    return r
+
+
+def drop_cls_rows(t, n_tok):
+    """[B * n_tok, D] -> the [B * (n_tok - 1), D] patch rows (token 0 of every image dropped)."""
+    return t.view(-1, n_tok, t.shape[-1])[:, 1:].reshape(-1, t.shape[-1])
+
+
+# The four token-LayerNorm launches of forward_body (csrc/ada_api.cu):
+LN_KINDS = {
+    "plain": dict(),                                             # norm1 of block 0
+    "norm2": dict(delta=True),                                   # norm2: x + attention branch, x not stored
+    "tap": dict(delta=True, delta2=True, write_x=True, tap=True),  # norm1 after a tapped block + the fused tap
+    "last": dict(delta=True, delta2=True, drop_cls=True),        # the last tap: patch rows only
+}
+# (D, B, n_tok, kind): every width (ViT-S / B / L / G) x every launch kind; B * n_tok is never a multiple of 8 (the
+# kernel walks rows from the last one, eight per block); n_tok 2 / 17 / 1370 = one patch, ViT-G at 56^2, ViT-S at 518^2.
+LN_ROWS = [
+    (384, 5, 2, "plain"), (384, 3, 17, "norm2"), (384, 2, 1370, "tap"), (384, 5, 2, "last"),
+    (768, 3, 17, "plain"), (768, 2, 1370, "norm2"), (768, 5, 2, "tap"), (768, 3, 17, "last"),
+    (1024, 2, 1370, "plain"), (1024, 5, 2, "norm2"), (1024, 3, 17, "tap"), (1024, 2, 1370, "last"),
+    (1536, 5, 2, "plain"), (1536, 3, 17, "norm2"), (1536, 2, 1370, "tap"), (1536, 3, 17, "last"),
+]
+
+
+def chk_layernorm_geo(D, B, n_tok, kind, seed=0):
+    """One token-LayerNorm launch (kind: a key of LN_KINDS, or such a dict of launch options): out (and the fused tap
+    out2) held to the fp64 bound of the fp32 stream (x + d) + d2 the kernel normalises; x afterwards bit-equal to that
+    stream when write_x is set and unchanged otherwise; the fused tap bit-equal to the separate tap pass; canaries around
+    out, out2 and x intact; d / d2 inside NaN guards; no unwritten (NaN) output row."""
+    torch, L, ops = _imports()
+    dev = "cuda"
+    t0 = time.time()
+    k = LN_KINDS[kind] if isinstance(kind, str) else kind
+    rows = B * n_tok
+    op = ln_operands(rows, D, seed, dev, deltas=k.get("delta", False))
+    x0 = op["x"]
+    guard = _guard_for(D)
+    gx = Guarded((rows, D), torch.float32, dev, guard)
+    gx.t.copy_(x0)
+    gd = {}
+    for nm in ("d", "d2"):
+        if k.get("delta" if nm == "d" else "delta2"):
+            gd[nm] = Guarded((rows, D), torch.bfloat16, dev, guard, fill=float("nan"))
+            gd[nm].t.copy_(op[nm])
+    xs = x0
+    if "d" in gd:
+        xs = xs + op["d"].float()
+    if "d2" in gd:
+        xs = xs + op["d2"].float()
+    patch_rows = B * (n_tok - 1)
+    go = Guarded((patch_rows if k.get("drop_cls") else rows, D), torch.bfloat16, dev, guard)
+    go2 = Guarded((patch_rows, D), torch.bfloat16, dev, guard) if k.get("tap") else None
+    ops.layernorm(gx.t, op["w"], op["b"], LN_EPS, n_tok, bool(k.get("drop_cls")), delta=gd["d"].t if "d" in gd else None,
+                  write_x=bool(k.get("write_x")), delta2=gd["d2"].t if "d2" in gd else None,
+                  tap_w=op["w2"] if go2 else None, tap_b=op["b2"] if go2 else None, out=go.t, out2=go2.t if go2 else None)
+    torch.cuda.synchronize()
+    i32 = torch.int32
+    res = {}
+    ref, bound = ln_ref64(drop_cls_rows(xs, n_tok) if k.get("drop_cls") else xs, op["w"], op["b"])
+    res["out"] = ln_verdict(go.t, ref, bound)
+    ok = res["out"]["ok"]
+    res["err_bound"] = res["out"]["err_bound"]
+    res["x_as_expected"] = bool(torch.equal(gx.t.view(i32), (xs if k.get("write_x") else x0).view(i32)))
+    canaries = go.canaries_intact() and gx.canaries_intact()
+    if go2 is not None:
+        ref2, bound2 = ln_ref64(drop_cls_rows(xs, n_tok), op["w2"], op["b2"])
+        res["tap"] = ln_verdict(go2.t, ref2, bound2)
+        res["err_bound"] = max(res["err_bound"], res["tap"]["err_bound"])
+        canaries = canaries and go2.canaries_intact()
+        sep = Guarded((patch_rows, D), torch.bfloat16, dev, guard)  # the separate tap pass (what the last block uses)
+        ops.layernorm(x0.clone(), op["w2"], op["b2"], LN_EPS, n_tok, True, delta=gd["d"].t, write_x=False,
+                      delta2=gd["d2"].t, out=sep.t)
+        torch.cuda.synchronize()
+        res["tap_same_bits_as_separate_pass"] = bool(torch.equal(sep.t.view(torch.int16), go2.t.view(torch.int16)))
+        ok = ok and res["tap"]["ok"] and res["tap_same_bits_as_separate_pass"] and sep.canaries_intact()
+    res["canaries_ok"] = bool(canaries)
+    res["deltas_untouched"] = all(bool(torch.equal(gd[nm].t.view(torch.int16), op[nm].view(torch.int16))) for nm in gd)
+    res["ok"] = bool(ok and res["x_as_expected"] and res["canaries_ok"] and res["deltas_untouched"])
+    res["run_sec"] = round(time.time() - t0, 2)
+    return res
+
+
+# Channel LayerNorm + ReLU: 48 / 256 (the conv-epilogue widths, run stand-alone here) and every width the model runs
+# through channel_ln_relu_kernel (C > 256: 384 ViT-S, 512, 768 ViT-B, 1024, 1536); 384 and 768 leave the last 32-lane
+# round of a multi-group instantiation (<2, true, 2>, <4, false, 1>) partly / wholly idle.
+CHLN_WIDTHS = (48, 256, 384, 512, 768, 1024, 1536)
+
+
+def chln_pixels(C, sms):
+    """A pixel count for which the persistent warps of launch_channel_ln_relu walk more than two grid strides and the last
+    stride is ragged: stride = sms * 8 blocks * 8 warps * pixels per warp."""
+    pix = 4 if C <= 256 else 2 if C <= 512 else 1
+    return 2 * sms * 64 * pix + 8 * pix * 37 + 5
+
+
+def chk_channel_ln_geo(C, seed=0, pixels=None):
+    """Channel LayerNorm + ReLU on NHWC bf16 pixels of every row kind: fp64 bound, input (in a NaN-guarded buffer)
+    unchanged, output canaries intact and no unwritten pixel; in place gives the same bits."""
+    torch, L, ops = _imports()
+    dev = "cuda"
+    t0 = time.time()
+    P = pixels or chln_pixels(C, torch.cuda.get_device_properties(0).multi_processor_count)
+    op = ln_operands(P, C, seed, dev)
+    x = op["x"].bfloat16()
+    guard = _guard_for(C)
+    gx = Guarded((P, C), torch.bfloat16, dev, guard, fill=float("nan"))
+    gx.t.copy_(x)
+    go = Guarded((P, C), torch.bfloat16, dev, guard)
+    ops.channel_ln_relu(gx.t, op["w"], op["b"], out=go.t)
+    torch.cuda.synchronize()
+    ref, bound = ln_ref64(x, op["w"], op["b"], relu=True)
+    res = ln_verdict(go.t, ref, bound)
+    res["pixels"] = P
+    res["canaries_ok"] = go.canaries_intact()
+    res["input_untouched"] = bool(torch.equal(gx.t.view(torch.int16), x.view(torch.int16)))
+    ops.channel_ln_relu(gx.t, op["w"], op["b"], out=gx.t)  # in place, as the model runs it
+    torch.cuda.synchronize()
+    res["in_place_same_bits"] = bool(torch.equal(gx.t.view(torch.int16), go.t.view(torch.int16)))
+    res["ok"] = bool(res["ok"] and res["canaries_ok"] and res["input_untouched"] and res["in_place_same_bits"])
+    res["run_sec"] = round(time.time() - t0, 2)
+    return res
+
+
+def _all_ok(*results):
+    """Several checks under one name: ok when all are."""
+    return {"ok": all(r["ok"] for r in results), "err_bound": max(r.get("err_bound", 0.0) for r in results),
+            "parts": list(results)}
+
+
+# The attention / LayerNorm checks of the first bring-up, by their original names: each shape and input of theirs, now held
+# to the fp64 bounds above (one kernel per attention row; bit-identity of the kernels for the impls_agree rows).
+#   name: (B, N, heads, input mode of att_operands)
+ATT_IMPL_ROWS = {
+    "small": (1, 128, 1, "rand"), "ragged": (1, 200, 2, "rand"), "1370": (2, 1370, 6, "rand"),
+    "rescale": (1, 1370, 2, "grow"), "5477": (1, 5477, 2, "rand"),
+    # persistent kernel: several work units per CTA, full (two query tiles) and short (one tile) units interleaved
+    "multiunit_1370": (4, 1370, 16, "rand"), "multiunit_300": (8, 300, 16, "rand"), "multiunit_128": (10, 128, 16, "rand"),
+    "multiunit_rescale": (3, 700, 16, "grow"),
+}
+ATT_AGREE_ROWS = {"1370": (3, 1370, 16, "rand"), "rescale": (2, 700, 16, "grow"), "5477": (1, 5477, 4, "rand")}
+
 CHECKS = {
     "gemm_resid_f32": lambda: chk_gemm_resid_f32(1370 * 3, 1024, 1024),
     "gemm_resid_f32_cg2": lambda: chk_gemm_resid_f32(1370 * 3, 1024, 4096, cg=2),
@@ -826,35 +1101,10 @@ CHECKS = {
     "convT_k4_c64_w5_tma": lambda: chk_convT(4, 64, 64, B=3, H=7, W=5, pix=True),
     "convT_k2_c128_w49_tma": lambda: chk_convT(2, 192, 128, B=1, H=37, W=49, pix=True),
     "convT_k2_c256_linear": lambda: chk_convT(2, 256, 256),
-    # both attention kernels on every shape (impl 0 = attention.cuh, 1 / 2 = attention2.cuh one / two threads per row), then the auto-selected one
-    **{f"attention{i}_small": (lambda i=i: chk_attention(1, 128, 1, impl=i)) for i in (0, 1, 2)},
-    **{f"attention{i}_ragged": (lambda i=i: chk_attention(1, 200, 2, impl=i)) for i in (0, 1, 2)},
-    **{f"attention{i}_1370": (lambda i=i: chk_attention(2, 1370, 6, impl=i)) for i in (0, 1, 2)},
-    **{f"attention{i}_rescale": (lambda i=i: chk_attention(1, 1370, 2, grow=True, impl=i)) for i in (0, 1, 2)},
-    **{f"attention{i}_5477": (lambda i=i: chk_attention(1, 5477, 2, impl=i)) for i in (0, 1, 2)},
-    # persistent kernel: several work units per CTA, full (two query tiles) and short (one tile) units interleaved
-    **{f"attention{i}_multiunit_1370": (lambda i=i: chk_attention(4, 1370, 16, impl=i)) for i in (0, 1, 2)},
-    **{f"attention{i}_multiunit_300": (lambda i=i: chk_attention(8, 300, 16, impl=i)) for i in (0, 1, 2)},
-    **{f"attention{i}_multiunit_128": (lambda i=i: chk_attention(10, 128, 16, impl=i)) for i in (0, 1, 2)},
-    **{f"attention{i}_multiunit_rescale": (lambda i=i: chk_attention(3, 700, 16, grow=True, impl=i)) for i in (0, 1, 2)},
-    "attention_auto_b32": lambda: chk_attention(32, 1370, 16),
-    "attention_impls_agree_1370": lambda: chk_attention_impls_agree(3, 1370, 16),
-    "attention_impls_agree_rescale": lambda: chk_attention_impls_agree(2, 700, 16, grow=True),
-    "attention_impls_agree_5477": lambda: chk_attention_impls_agree(1, 5477, 4),
-    "layernorm_384": lambda: chk_layernorm(384, False),
-    "layernorm_1024_drop": lambda: chk_layernorm(1024, True),
-    "layernorm_1536": lambda: chk_layernorm(1536, False),
-    "layernorm_delta": chk_layernorm_delta,
-    "layernorm_tap_fused": chk_layernorm_tap,
-    "channel_ln_48": lambda: chk_channel_ln(48),
-    "channel_ln_1024": lambda: chk_channel_ln(1024),
     "upsample_19_37": lambda: chk_upsample(19, 37),
     "upsample_37_74": lambda: chk_upsample(37, 74),
     "upsample_148_296_c256": lambda: chk_upsample(148, 296, 256),
     "upsample_40_70_c128": lambda: chk_upsample(40, 70, 128),   # not a 2x map: strips cross source rows irregularly
-    "channel_ln_256": lambda: chk_channel_ln(256),
-    "channel_ln_512": lambda: chk_channel_ln(512),
-    "channel_ln_1536": lambda: chk_channel_ln(1536),
     "fused_tail_5x7": lambda: chk_fused_tail(5, 7),
     "fused_tail_9x9": lambda: chk_fused_tail(9, 9),
     "tail_mma_5x7_c64": lambda: chk_tail_mma(5, 7, 64),
@@ -877,6 +1127,24 @@ CHECKS = {
                                                               (0, 16, 31))) for h in (148, 74, 37, 19)},
     "conv_geo_bench_s2_37": lambda: chk_conv_geo_bench(32, 19, 19, ("h_s2_bias",), (0, 16, 31)),
     **{f"gemm_tiles_{k}": (lambda k=k: chk_gemm_tiles(k)) for k in GEMM_TILES},
+    # both attention kernels (impl 0 = attention.cuh, 1 / 2 = attention2.cuh one / two threads per row), then the default
+    **{f"attention{i}_{n}": (lambda i=i, r=r: chk_attention_geo(*r[:3], (r[3],), impls=(i,)))
+       for n, r in ATT_IMPL_ROWS.items() for i in (0, 1, 2)},
+    "attention_auto_b32": lambda: chk_attention_geo(32, 1370, 16, ("rand",), ((0, 0), (16, 7), (31, 15)), impls=(-1,)),
+    **{f"attention_impls_agree_{n}": (lambda r=r: chk_attention_geo(*r[:3], (r[3],), seed=15)) for n, r in ATT_AGREE_ROWS.items()},
+    "layernorm_384": lambda: chk_layernorm_geo(384, 3, 50, "plain", seed=6),
+    "layernorm_1024_drop": lambda: chk_layernorm_geo(1024, 3, 50, dict(drop_cls=True), seed=6),
+    "layernorm_1536": lambda: chk_layernorm_geo(1536, 3, 50, "plain", seed=6),
+    "layernorm_delta": lambda: _all_ok(chk_layernorm_geo(1024, 300, 1, dict(delta=True, write_x=True), seed=16),
+                                       chk_layernorm_geo(1024, 300, 1, "norm2", seed=16),
+                                       chk_layernorm_geo(1024, 300, 1, dict(delta=True, delta2=True, write_x=True), seed=16)),
+    "layernorm_tap_fused": lambda: chk_layernorm_geo(1024, 3, 50, "tap", seed=26),
+    **{f"channel_ln_{c}": (lambda c=c: chk_channel_ln_geo(c, seed=7, pixels=2 * 9 * 11)) for c in (48, 256, 512, 1024, 1536)},
+    # attention at every ragged residue, tile count and head count against fp64, all kernels bit-identical
+    **{f"attention_geo_{r[0]}x{r[1]}x{r[2]}": (lambda r=r, i=i: chk_attention_geo(*r, seed=i)) for i, r in enumerate(ATT_ROWS)},
+    # token LayerNorm: every width x every launch kind of the encoder; channel LayerNorm + ReLU at every width
+    **{f"ln_geo_{r[0]}_{r[3]}": (lambda r=r, i=i: chk_layernorm_geo(*r, seed=i)) for i, r in enumerate(LN_ROWS)},
+    **{f"ln_geo_channel_{c}": (lambda c=c, i=i: chk_channel_ln_geo(c, seed=i)) for i, c in enumerate(CHLN_WIDTHS)},
 }
 
 
