@@ -683,6 +683,8 @@ static void launch_upsample(const __nv_bfloat16* in, __nv_bfloat16* out, int B, 
 
 static void launch_tail_gather(const __half* V, const float* bias2, const float* aux, float* out, int B, int Hl,
                                int Wl, int H, int W, int sigmoid, cudaStream_t st) {
+  // other geometries can need a low-resolution patch of more than 12 x 12 and trap (tests/test_head_check_cpu.py)
+  ADA_REQUIRE(Hl * 14 == H * 8 && Wl * 14 == W * 8, "tail_gather: 8h -> 14h geometry");
   static std::atomic<uint64_t> attr_done{0};
   ensure_smem_attr(tail_gather_kernel, kTailSmemBytes, attr_done);
   dim3 grid((W + kTailTile - 1) / kTailTile, (H + kTailTile - 1) / kTailTile, B);

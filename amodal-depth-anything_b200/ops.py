@@ -96,16 +96,23 @@ def channel_ln_relu(x_nhwc, w, b, eps=1e-6, out=None):
     return out
 
 
-def upsample(x_nhwc, Ho, Wo):
+def upsample(x_nhwc, Ho, Wo, out=None):
+    """out: bf16 [B, Ho, Wo, C] to store into (allocated when None)."""
     B, Hi, Wi, C = x_nhwc.shape
-    out = torch.empty(B, Ho, Wo, C, dtype=torch.bfloat16, device=x_nhwc.device)
+    if out is None:
+        out = torch.empty(B, Ho, Wo, C, dtype=torch.bfloat16, device=x_nhwc.device)
+    assert out.shape == (B, Ho, Wo, C) and out.dtype == torch.bfloat16 and out.is_contiguous()
     _call(x_nhwc, L.load().ada_op_upsample, _p(x_nhwc), _p(out), B, Hi, Wi, Ho, Wo, C)
     return out
 
 
-def patch_gather(rgb, guides, Kpad):
+def patch_gather(rgb, guides, Kpad, out=None):
+    """out: bf16 [B * (H // 14) * (W // 14), Kpad] to store into (allocated and zeroed when None); the kernel leaves the
+    columns past the patch rows' C * 196 elements as they were."""
     B, _, H, W = rgb.shape
-    out = torch.zeros(B * (H // 14) * (W // 14), Kpad, dtype=torch.bfloat16, device=rgb.device)
+    if out is None:
+        out = torch.zeros(B * (H // 14) * (W // 14), Kpad, dtype=torch.bfloat16, device=rgb.device)
+    assert out.shape == (B * (H // 14) * (W // 14), Kpad) and out.dtype == torch.bfloat16 and out.is_contiguous()
     n = len(guides)
     ptrs = (ctypes.c_void_p * max(n, 1))(*[g.data_ptr() for g in guides])
     chs = (ctypes.c_int32 * max(n, 1))(*[g.shape[1] for g in guides])
@@ -141,10 +148,12 @@ def pack_tail_taps(w):
     return out
 
 
-def tail_gather(V, bias2, aux, H, W, sigmoid=True):
-    """V: NHWC fp16 [B,Hl,Wl,288] -> fp32 [B,H,W]."""
+def tail_gather(V, bias2, aux, H, W, sigmoid=True, out=None):
+    """V: NHWC fp16 [B,Hl,Wl,288] -> fp32 [B,H,W] (out: stored into when given)."""
     B, Hl, Wl, _ = V.shape
-    out = torch.empty(B, H, W, dtype=torch.float32, device=V.device)
+    if out is None:
+        out = torch.empty(B, H, W, dtype=torch.float32, device=V.device)
+    assert out.shape == (B, H, W) and out.dtype == torch.float32 and out.is_contiguous()
     _call(V, L.load().ada_op_tail_gather, _p(V), _p(bias2), _p(aux), _p(out), B, Hl, Wl, H, W, int(sigmoid))
     return out
 
@@ -158,10 +167,13 @@ def pack_tail_mma(w):
     return out
 
 
-def tail_mma(Lmap, wpk, bias2, aux, H, W, sigmoid=1):
-    """Lmap: NHWC fp16 [B,Hl,Wl,C] (output_conv1 map) -> fp32 [B,H,W]: upsample + output_conv2 in one kernel."""
+def tail_mma(Lmap, wpk, bias2, aux, H, W, sigmoid=1, out=None):
+    """Lmap: NHWC fp16 [B,Hl,Wl,C] (output_conv1 map) -> fp32 [B,H,W]: upsample + output_conv2 in one kernel (out: stored
+    into when given)."""
     B, Hl, Wl, C = Lmap.shape
-    out = torch.empty(B, H, W, dtype=torch.float32, device=Lmap.device)
+    if out is None:
+        out = torch.empty(B, H, W, dtype=torch.float32, device=Lmap.device)
+    assert out.shape == (B, H, W) and out.dtype == torch.float32 and out.is_contiguous()
     _call(Lmap, L.load().ada_op_tail_mma, _p(Lmap), _p(wpk), _p(bias2), _p(aux), _p(out), B, Hl, Wl, H, W, C, int(sigmoid))
     return out
 

@@ -136,33 +136,21 @@ def chk_conv(B, H, W, Cin, Cout, mode, cg=0):
 
 
 def chk_convT(ks, Cin=96, Cout=96, B=2, H=37, W=37, pix=False):
-    """pix: A operand on 8x16 pixel tiles, pixel shuffle stored through 5-D TMA boxes (Cin, Cout % 64 == 0)."""
+    """pix: A operand on 8x16 pixel tiles, pixel shuffle stored through 5-D TMA boxes (Cin, Cout % 64 == 0). Held to the fp64
+    bound of convT_run."""
     torch, L, ops = _imports()
     g = torch.Generator(device="cuda").manual_seed(4)
     x = torch.randn(B, Cin, H, W, generator=g, device="cuda").bfloat16()
     w = torch.randn(Cin, Cout, ks, ks, generator=g, device="cuda") * 0.1
     bias = torch.randn(Cout, generator=g, device="cuda") * 0.1
-    ref = torch.nn.functional.conv_transpose2d(x.float(), w.bfloat16().float(), bias, stride=ks)
-    x_nhwc = x.permute(0, 2, 3, 1).contiguous()
-    wp = ops.pack_convT(w, ks)
-    out = torch.zeros(B, H * ks, W * ks, Cout, dtype=torch.bfloat16, device="cuda")
-    if pix:
-        ops.gemm(x_nhwc, wp, conv=(B, H, W, Cin), conv_taps=1, N=ks * ks * Cout, epi=L.EPI_CONVT, bias=bias, out_bf16=out, ks=ks,
-                 cout=Cout)
-    else:
-        ops.gemm(x_nhwc.reshape(B * H * W, Cin), wp, epi=L.EPI_CONVT, bias=bias, out_bf16=out, ks=ks, cout=Cout, H=H, W=W)
-    torch.cuda.synchronize()
-    return _cmp("convT", out.permute(0, 3, 1, 2), ref, 3e-2, 1e-2)
+    return convT_run({"x": x.permute(0, 2, 3, 1).contiguous(), "w": w.bfloat16().float(), "b": bias}, ks, pix)
 
 
 def chk_upsample(Hi, Ho, C=64):
     torch, L, ops = _imports()
     g = torch.Generator(device="cuda").manual_seed(8)
     x = torch.randn(2, Hi, Hi, C, generator=g, device="cuda").bfloat16()
-    out = ops.upsample(x, Ho, Ho)
-    torch.cuda.synchronize()
-    ref = torch.nn.functional.interpolate(x.float().permute(0, 3, 1, 2), (Ho, Ho), mode="bilinear", align_corners=True)
-    return _cmp("up", out.permute(0, 3, 1, 2), ref, 2e-2, 1e-2)
+    return upsample_run(x, Ho, Ho)
 
 
 def chk_fused_tail(gh, gw):
@@ -216,16 +204,7 @@ def chk_patch_gather():
     rgb = torch.rand(B, 3, H, W, generator=g, device="cuda")
     m = torch.rand(B, 1, H, W, generator=g, device="cuda") * 2 - 1
     o = torch.rand(B, 1, H, W, generator=g, device="cuda") * 2 - 1
-    out = ops.patch_gather(rgb, [m, o], 1024)
-    torch.cuda.synchronize()
-    mean = torch.tensor([0.485, 0.456, 0.406], device="cuda").view(1, 3, 1, 1)
-    std = torch.tensor([0.229, 0.224, 0.225], device="cuda").view(1, 3, 1, 1)
-    x = torch.cat([(rgb - mean) / std, m, o], 1)
-    ref = torch.nn.functional.unfold(x, 14, stride=14).transpose(1, 2).reshape(B * (H // 14) * (W // 14), 5 * 196)
-    r = _cmp("gather", out[:, :980], ref, 1e-6, 2 ** -8)
-    r["pad_zero"] = bool((out[:, 980:] == 0).all().item())
-    r["ok"] = r["ok"] and r["pad_zero"]
-    return r
+    return patch_gather_run(rgb, [m, o], 1024)
 
 
 def chk_conv_s2(B, H, W, Cin, Cout):
@@ -1049,6 +1028,345 @@ def chk_channel_ln_geo(C, seed=0, pixels=None):
     return res
 
 
+# ---- DPT head bandwidth kernels: k = s transposed convs, bilinear upsample, patch gather
+#
+# Transposed convs (EPI_CONVT): every output is one bias plus a Ci-term dot product of bf16 operands accumulated in fp32 and
+# stored as bf16, so the conv error model above holds with S = conv_transpose2d(|x|, |w|) + |b|.
+def convT_operands(B, H, W, Ci, Co, ks, mode, seed, device="cpu"):
+    """x [B, H, W, Ci] bf16, w [Ci, Co, ks, ks] rounded to bf16 (held as fp32), b [Co] fp32. mode "rand": N(0, 1) inputs;
+    "onehot": pixel (b, y, x) is one-hot at channel (5 b + 3 y + x) mod Ci, so every output is a single weight
+    w[c, co, ky, kx] + b[co], and a pixel shuffle that swaps ky and kx, or picks the wrong image or channel slab, moves it by
+    O(1) instead of by rounding."""
+    import torch
+    g = torch.Generator(device=device).manual_seed(seed)
+    w = (torch.randn(Ci, Co, ks, ks, generator=g, device=device) / Ci ** 0.5).bfloat16().float()
+    b = torch.randn(Co, generator=g, device=device) * 0.1
+    if mode == "rand":
+        x = torch.randn(B, H, W, Ci, generator=g, device=device).bfloat16()
+    else:
+        assert mode == "onehot", mode
+        bi, yi, xi = torch.meshgrid(*(torch.arange(n, device=device) for n in (B, H, W)), indexing="ij")
+        x = torch.nn.functional.one_hot((5 * bi + 3 * yi + xi) % Ci, Ci).bfloat16()
+    return {"x": x, "w": w, "b": b}
+
+
+def convT_ref64(op, ks, imgs=None):
+    """fp64 reference of the k = s transposed conv on convT_operands-style op (any device) and its per-element bound:
+    (ref, bound) as [b, H ks, W ks, Co] over the images `imgs` (all if None)."""
+    import torch
+    F = torch.nn.functional
+    x = op["x"] if imgs is None else op["x"][list(imgs)]
+    xd, wd, bd = x.double().permute(0, 3, 1, 2), op["w"].double().to(x.device), op["b"].double().to(x.device)
+    ref = F.conv_transpose2d(xd, wd, bd, stride=ks).permute(0, 2, 3, 1)
+    S = F.conv_transpose2d(xd.abs(), wd.abs(), bd.abs(), stride=ks).permute(0, 2, 3, 1)
+    return ref, REL_BF16 * ref.abs() + REL_ACC * S
+
+
+def head_verdict(got, ref, bound):
+    """got / ref / bound of one head kernel: within the bound everywhere, no NaN."""
+    import torch
+    r = {"err_bound": err_over_bound(got, ref, bound), "nan": int(torch.isnan(got.float()).sum().item())}
+    r["ok"] = r["err_bound"] <= 1.0 and r["nan"] == 0
+    return r
+
+
+def _ref_device(work):
+    """Large fp64 references (work: their multiply-adds) run on the device, as conv_geo_bench_* does; small ones on the host."""
+    return "cuda" if work > 3e8 else "cpu"
+
+
+def convT_run(op, ks, pix, cg=0, ref_imgs=None):
+    """One transposed conv as forward_body launches it (pix: pixel-tile A operand and 5-D TMA stores, else linear A rows and
+    per-thread scatter), force_cg=cg: x inside a NaN guard of one image on either side, the output canary-guarded and
+    NaN-filled; fp64 bound on `ref_imgs` (all if None), no unwritten pixel, x unchanged, every image launched alone
+    bit-equal to the batch, and with cg = 2 bit-equal to single-CTA tiles."""
+    torch, L, ops = _imports()
+    dev = "cuda"
+    t0 = time.time()
+    x = op["x"]
+    B, H, W, Ci = x.shape
+    Co = op["w"].shape[1]
+    imgs = list(range(B)) if ref_imgs is None else list(ref_imgs)
+    gx = Guarded(tuple(x.shape), torch.bfloat16, dev, _guard_for(H * W * Ci), fill=float("nan"))
+    gx.t.copy_(x)
+    wp = ops.pack_convT(op["w"], ks)
+    b = op["b"].to(dev)
+
+    def launch(xin, c):
+        nb = xin.shape[0]
+        o = Guarded((nb, H * ks, W * ks, Co), torch.bfloat16, dev, _guard_for(H * W * ks * ks * Co))
+        if pix:
+            ops.gemm(xin, wp, conv=(nb, H, W, Ci), conv_taps=1, N=ks * ks * Co, epi=L.EPI_CONVT, bias=b, out_bf16=o.t, ks=ks,
+                     cout=Co, force_cg=c)
+        else:
+            ops.gemm(xin.reshape(nb * H * W, Ci), wp, epi=L.EPI_CONVT, bias=b, out_bf16=o.t, ks=ks, cout=Co, H=H, W=W,
+                     force_cg=c)
+        return o
+
+    out = launch(gx.t, cg)
+    torch.cuda.synchronize()
+    rd = _ref_device(2.0 * len(imgs) * H * W * Ci * Co * ks * ks)
+    ref, bound = convT_ref64({"x": x.to(rd), "w": op["w"].to(rd), "b": op["b"].to(rd)}, ks, imgs)
+    r = head_verdict(out.t[imgs].to(rd), ref, bound)
+    del ref, bound
+    r["nan_all"] = int(torch.isnan(out.t.float()).sum().item())
+    i16 = torch.int16
+    same = True
+    for i in range(B):
+        o1 = launch(gx.t[i:i + 1], 0)
+        same = same and bool(torch.equal(o1.t.view(i16), out.t[i:i + 1].view(i16))) and o1.canaries_intact()
+    r["batch_invariant"] = same
+    if cg == 2:
+        o2 = launch(gx.t, 1)
+        r["pair_invariant"] = bool(torch.equal(o2.t.view(i16), out.t.view(i16)))
+    else:
+        r["pair_invariant"] = True
+    torch.cuda.synchronize()
+    r["canaries_ok"] = out.canaries_intact()
+    r["input_untouched"] = bool(torch.equal(gx.t.view(i16), x.view(i16)))
+    r["ok"] = bool(r["ok"] and r["nan_all"] == 0 and r["batch_invariant"] and r["pair_invariant"] and r["canaries_ok"]
+                   and r["input_untouched"])
+    r["run_sec"] = round(time.time() - t0, 2)
+    return r
+
+
+# (ks, Ci, B, H, W, force_cg, ref_imgs): resize_layers[0] (k 4) and [1] (k 2) of every encoder, Co = Ci, on the path
+# forward_body takes (pixel tiles when Ci % 64 == 0, linear A rows otherwise). Widths ragged against the 16-pixel tile
+# (37, 49, 7, 5), exact (32) and 1 x 1. force_cg = 2 pairs CTAs where pick_bn gives 256-wide tiles (N = ks^2 Ci >= 768).
+# At 32 x 32, B = 4, Ci 256, k 4 the launcher pairs on its own: 4096 padded pixels either way, 16 x 16 = 256 pairs >= 148.
+CONVT_GEO_ROWS = [
+    (4, 48, 3, 37, 37, 0, None),      # ViT-S level 0 at 518^2 (linear)
+    (4, 48, 2, 7, 5, 0, None),        # ViT-S level 0 at 98 x 70
+    (4, 96, 2, 37, 49, 0, None),      # ViT-B level 0 at 518 x 686 (linear)
+    (4, 96, 5, 1, 1, 0, None),        # ViT-B level 0 at 14^2
+    (4, 256, 2, 37, 49, 0, None),     # ViT-L level 0 (pixel tiles)
+    (4, 256, 3, 1, 1, 0, None),       # ViT-L level 0 at 14^2
+    (4, 1536, 2, 5, 7, 0, None),      # ViT-G level 0 (guided, and the un-guided ViT-G of infer.py)
+    (4, 1536, 1, 4, 4, 0, None),      # ViT-G level 0 at 56^2
+    (2, 96, 2, 37, 37, 0, None),      # ViT-S level 1 (linear)
+    (2, 96, 3, 1, 1, 0, None),        # ViT-S level 1 at 14^2
+    (2, 192, 2, 37, 49, 0, None),     # ViT-B level 1 (pixel tiles)
+    (2, 192, 3, 7, 5, 0, None),       # ViT-B level 1 at 98 x 70
+    (2, 512, 2, 32, 32, 0, None),     # ViT-L level 1 at 448^2: whole 16-pixel tiles
+    (2, 1536, 2, 7, 5, 0, None),      # ViT-G level 1
+    (2, 1536, 2, 1, 1, 0, None),      # ViT-G level 1 at 14^2
+    (4, 256, 2, 32, 32, 2, None),     # CTA pairs, pixel tiles: bit-equal to single CTAs
+    (4, 256, 2, 37, 37, 2, None),
+    (2, 512, 1, 37, 37, 2, None),
+    (4, 48, 2, 37, 37, 2, None),      # CTA pairs, linear A rows
+    (4, 256, 4, 32, 32, 0, None),     # the launcher's own pairing (ViT-L at 448^2, batch 4)
+    (4, 256, 32, 37, 37, 0, (0, 16, 31)),  # the benchmark's ViT-L launches: 518^2, batch 32
+    (2, 512, 32, 37, 37, 0, (0, 16, 31)),
+]
+
+
+def chk_convT_geo(ks, Ci, B, H, W, cg=0, ref_imgs=None, seed=0, modes=("rand", "onehot")):
+    torch, L, ops = _imports()
+    parts = {}
+    for mi, mode in enumerate(modes):
+        op = convT_operands(B, H, W, Ci, Ci, ks, mode, seed * 8 + mi, device="cuda")
+        parts[mode] = convT_run(op, ks, Ci % 64 == 0, cg, ref_imgs)
+        del op
+    return {"ok": all(p["ok"] for p in parts.values()), "err_bound": max(p["err_bound"] for p in parts.values()),
+            "modes": parts, "run_sec": round(sum(p["run_sec"] for p in parts.values()), 2)}
+
+
+# Bilinear upsample (align_corners=True). The source coordinates are ATen's, in fp32 as upsample_bilinear_kernel computes
+# them: scale = (in - 1) / (out - 1), src = scale * dst, i0 = (int) src, i1 = i0 + (i0 < in - 1), l = src - i0 (exact); the
+# reference interpolates with weights l and 1 - l in fp64 (tests/test_head_check_cpu.py pins these weights to
+# F.interpolate). Error model: the kernel forms 1 - l in fp32 (relative error <= 2^-24: exact for l >= 1/2), then per pass
+# two products and a sum in fp32 (three roundings), horizontally and then vertically: at most 6 units of 2^-24 relative to
+# sum w |corner| to first order, held to UP_C = 8. The bf16 store adds 2^-8 |ref|.
+UP_C = 8
+
+
+def up_coords(n_in, n_out):
+    """(i0, i1, l) per output index: ATen's align_corners=True source coordinates in fp32 (numpy int64 / fp64 arrays)."""
+    import numpy as np
+    scale = np.float32(n_in - 1) / np.float32(n_out - 1) if n_out > 1 else np.float32(0.0)
+    src = (scale * np.arange(n_out, dtype=np.float32)).astype(np.float32)
+    i0 = src.astype(np.int64)
+    i1 = i0 + (i0 < n_in - 1)
+    return i0, i1, (src - i0.astype(np.float32)).astype(np.float64)
+
+
+def up_matrix(n_in, n_out, device="cpu"):
+    """[n_out, n_in] fp64 interpolation weights of up_coords."""
+    import torch
+    i0, i1, lam = up_coords(n_in, n_out)
+    A = torch.zeros(n_out, n_in, dtype=torch.float64)
+    r = torch.arange(n_out)
+    lam = torch.from_numpy(lam)
+    A.index_put_((r, torch.from_numpy(i0)), 1.0 - lam, accumulate=True)
+    A.index_put_((r, torch.from_numpy(i1)), lam, accumulate=True)
+    return A.to(device)
+
+
+def up_ref64(x, Ho, Wo):
+    """fp64 bilinear of NHWC x (any device) to (Ho, Wo) and the per-element bound of the model above: (ref, bound)."""
+    import torch
+    Ah, Aw = up_matrix(x.shape[1], Ho, x.device), up_matrix(x.shape[2], Wo, x.device)
+    xd = x.double()
+    ref = torch.einsum("pw,bowc->bopc", Aw, torch.einsum("oh,bhwc->bowc", Ah, xd))
+    S = torch.einsum("pw,bowc->bopc", Aw, torch.einsum("oh,bhwc->bowc", Ah, xd.abs()))
+    return ref, REL_BF16 * ref.abs() + UP_C * 2.0 ** -24 * S
+
+
+def up_operands(B, Hi, Wi, C, mode, seed, device="cpu"):
+    """NHWC bf16 input. "rand": N(0, 1); "ramp": source row y of image b is offset by 100 ((3 y + 2 b) mod 5 - 2) on top of
+    N(0, 1), so neighbouring rows differ by at least 100x the spread inside a row: reading the wrong source row, or a stale
+    row across a strip boundary, misses the bound by orders of magnitude."""
+    import torch
+    g = torch.Generator(device=device).manual_seed(seed)
+    x = torch.randn(B, Hi, Wi, C, generator=g, device=device)
+    if mode == "ramp":
+        y, b = torch.arange(Hi, device=device).view(1, Hi, 1, 1), torch.arange(B, device=device).view(B, 1, 1, 1)
+        x = x + 100.0 * ((3 * y + 2 * b) % 5 - 2).float()
+    else:
+        assert mode == "rand", mode
+    return x.bfloat16()
+
+
+def upsample_run(x, Ho, Wo, ref_imgs=None):
+    """One upsample launch: x inside a NaN guard of one image on either side, output canary-guarded and NaN-filled; fp64
+    bound on `ref_imgs` (all if None), no unwritten pixel, x unchanged, every image launched alone bit-equal to the batch."""
+    torch, L, ops = _imports()
+    dev = "cuda"
+    t0 = time.time()
+    B, Hi, Wi, C = x.shape
+    imgs = list(range(B)) if ref_imgs is None else list(ref_imgs)
+    gx = Guarded(tuple(x.shape), torch.bfloat16, dev, _guard_for(Hi * Wi * C), fill=float("nan"))
+    gx.t.copy_(x)
+
+    def launch(xin):
+        o = Guarded((xin.shape[0], Ho, Wo, C), torch.bfloat16, dev, _guard_for(Ho * Wo * C))
+        ops.upsample(xin, Ho, Wo, out=o.t)
+        return o
+
+    out = launch(gx.t)
+    torch.cuda.synchronize()
+    rd = _ref_device(2.0 * len(imgs) * Ho * C * (Hi * Wi + Wo * Wi))
+    ref, bound = up_ref64(x[imgs].to(rd), Ho, Wo)
+    r = head_verdict(out.t[imgs].to(rd), ref, bound)
+    del ref, bound
+    r["nan_all"] = int(torch.isnan(out.t.float()).sum().item())
+    i16 = torch.int16
+    same = True
+    for i in range(B):
+        o1 = launch(gx.t[i:i + 1])
+        same = same and bool(torch.equal(o1.t.view(i16), out.t[i:i + 1].view(i16))) and o1.canaries_intact()
+    torch.cuda.synchronize()
+    r["batch_invariant"] = same
+    r["canaries_ok"] = out.canaries_intact()
+    r["input_untouched"] = bool(torch.equal(gx.t.view(i16), x.view(i16)))
+    r["ok"] = bool(r["ok"] and r["nan_all"] == 0 and r["batch_invariant"] and r["canaries_ok"] and r["input_untouched"])
+    r["run_sec"] = round(time.time() - t0, 2)
+    return r
+
+
+def up_maps(gh, gw):
+    """The four maps forward_body upsamples at patch grid gh x gw (refinenet4..1): down2(g) -> g, g -> 2g, 2g -> 4g,
+    4g -> 8g, as (Hi, Wi, Ho, Wo)."""
+    d2 = lambda n: (n - 1) // 2 + 1  # noqa: E731
+    return [(d2(gh), d2(gw), gh, gw)] + [(gh << k, gw << k, gh << (k + 1), gw << (k + 1)) for k in range(3)]
+
+
+# (gh, gw) per width F (ViT-S / B / L / G): gh = 1 gives Ho = 1 and Wo = 1 (scale 0); 5 gives maps of fewer than 16 rows and
+# heights that are not multiples of 16 (the last strip ragged); 9 x 7 non-square maps; 37 the 518^2 maps. F = 384 has 48
+# channel groups, not a power of two (the division path of the kernel's index math).
+UP_GRIDS = ((1, 1), (4, 4), (5, 5), (9, 7), (37, 37))
+UP_WIDTHS = (64, 128, 256, 384)
+
+
+def chk_upsample_geo(C, maps, B, ref_imgs=None, seed=0, modes=("rand", "ramp")):
+    parts = {}
+    for mi, (Hi, Wi, Ho, Wo) in enumerate(maps):
+        for mj, mode in enumerate(modes):
+            x = up_operands(B, Hi, Wi, C, mode, seed * 64 + mi * 8 + mj, device="cuda")
+            parts[f"{Hi}x{Wi}->{Ho}x{Wo}_{mode}"] = upsample_run(x, Ho, Wo, ref_imgs)
+            del x
+    return {"ok": all(p["ok"] for p in parts.values()), "err_bound": max(p["err_bound"] for p in parts.values()),
+            "maps": parts, "run_sec": round(sum(p["run_sec"] for p in parts.values()), 2)}
+
+
+# Patch gather: exactly specified, so checked bit for bit: ((x - mean) / std) in fp32 (RGB planes; guide planes pass
+# through as (x - 0) / 1), rounded to bf16, in the K order c * 196 + ky * 14 + kx of the patch-embed weight.
+PG_MEAN, PG_STD = (0.485, 0.456, 0.406), (0.229, 0.224, 0.225)
+
+
+def patch_gather_expected(rgb, guides, mean=PG_MEAN, std=PG_STD):
+    """[B * ph * pw, C * 196] bf16 on the CPU: what patch_gather_kernel must store, bit for bit."""
+    import torch
+    m = torch.tensor(mean, dtype=torch.float32).view(1, 3, 1, 1)
+    s = torch.tensor(std, dtype=torch.float32).view(1, 3, 1, 1)
+    x = torch.cat([(rgb.cpu() - m) / s] + [g.cpu() for g in guides], 1)
+    B, C, H, W = x.shape
+    ph, pw = H // 14, W // 14
+    x = x[:, :, :ph * 14, :pw * 14].reshape(B, C, ph, 14, pw, 14).permute(0, 2, 4, 1, 3, 5)
+    return x.reshape(B * ph * pw, C * 196).bfloat16()
+
+
+PG_SENTINEL = -3.0  # K-padding columns start as this and must keep it
+
+
+def patch_gather_run(rgb, guides, Kpad=None):
+    """One patch gather (normalize = 1, the path ada_op_patch_gather runs): image and guides inside NaN guards of one image
+    on either side, output canary-guarded with its patch columns NaN and its K padding PG_SENTINEL; the patch columns
+    bit-equal to patch_gather_expected, the padding and the inputs unchanged."""
+    torch, L, ops = _imports()
+    dev = "cuda"
+    t0 = time.time()
+    B, _, H, W = rgb.shape
+    K = (3 + sum(g.shape[1] for g in guides)) * 196
+    Kpad = Kpad or (K + 63) // 64 * 64
+    rows = B * (H // 14) * (W // 14)
+    gin = []
+    for t in [rgb] + list(guides):
+        gt = Guarded(tuple(t.shape), torch.float32, dev, _guard_for(t[0].numel()), fill=float("nan"))
+        gt.t.copy_(t)
+        gin.append(gt)
+    go = Guarded((rows, Kpad), torch.bfloat16, dev, _guard_for(Kpad), body=PG_SENTINEL)
+    go.t[:, :K] = float("nan")
+    ops.patch_gather(gin[0].t, [g.t for g in gin[1:]], Kpad, out=go.t)
+    torch.cuda.synchronize()
+    i16 = torch.int16
+    got = go.t.cpu()
+    exp = patch_gather_expected(rgb, guides)
+    r = {"bit_exact": bool(torch.equal(got[:, :K].view(i16), exp.view(i16)))}
+    r["mismatches"] = int((got[:, :K].view(i16) != exp.view(i16)).sum().item())
+    r["padding_untouched"] = bool((got[:, K:] == PG_SENTINEL).all().item())
+    r["canaries_ok"] = go.canaries_intact()
+    r["inputs_untouched"] = all(bool(torch.equal(g.t.view(torch.int32), t.view(torch.int32)))
+                                for g, t in zip(gin, [rgb] + list(guides)))
+    r["ok"] = bool(r["bit_exact"] and r["padding_untouched"] and r["canaries_ok"] and r["inputs_untouched"])
+    r["err_bound"] = 0.0
+    r["run_sec"] = round(time.time() - t0, 2)
+    return r
+
+
+# (B, H, W, guide channels per guide tensor): guide channels 0 (un-guided), 2 (mask + observation), 4 and 5; patches per
+# row 1, 5, 32, 33 (32 + 1), 37 (518: 32 + 5 in two blocks of 19 / 18) and 74 (1036: 25 + 25 + 24); the benchmark's batch.
+PG_ROWS = [
+    (3, 28, 14, ()),
+    (2, 42, 70, (1, 1)),
+    (2, 28, 448, (1, 3)),
+    (2, 14, 462, (3, 1, 1)),
+    (3, 28, 518, ()),
+    (2, 28, 518, (1, 1)),
+    (1, 28, 1036, (1, 1)),
+    (1, 14, 1036, (2, 3)),
+    (32, 518, 518, (1, 1)),
+]
+
+
+def chk_patch_gather_geo(B, H, W, guide_ch, seed=0):
+    import torch
+    g = torch.Generator(device="cuda").manual_seed(seed)
+    rgb = torch.rand(B, 3, H, W, generator=g, device="cuda")
+    guides = [torch.rand(B, c, H, W, generator=g, device="cuda") * 2 - 1 for c in guide_ch]
+    return patch_gather_run(rgb, guides)
+
+
 def _all_ok(*results):
     """Several checks under one name: ok when all are."""
     return {"ok": all(r["ok"] for r in results), "err_bound": max(r.get("err_bound", 0.0) for r in results),
@@ -1145,6 +1463,15 @@ CHECKS = {
     # token LayerNorm: every width x every launch kind of the encoder; channel LayerNorm + ReLU at every width
     **{f"ln_geo_{r[0]}_{r[3]}": (lambda r=r, i=i: chk_layernorm_geo(*r, seed=i)) for i, r in enumerate(LN_ROWS)},
     **{f"ln_geo_channel_{c}": (lambda c=c, i=i: chk_channel_ln_geo(c, seed=i)) for i, c in enumerate(CHLN_WIDTHS)},
+    # DPT head: transposed convs, the four upsample maps at every width, patch gather, against fp64 / exact references
+    **{f"convT_geo_k{r[0]}_c{r[1]}_{r[3]}x{r[4]}_b{r[2]}" + (f"_cg{r[5]}" if r[5] else ""): (lambda r=r, i=i: chk_convT_geo(*r, seed=i))
+       for i, r in enumerate(CONVT_GEO_ROWS)},
+    **{f"upsample_geo_c{c}_{gh}x{gw}": (lambda c=c, gh=gh, gw=gw, i=i: chk_upsample_geo(c, up_maps(gh, gw), 2 if gh > 9 else 3, seed=i))
+       for i, (c, (gh, gw)) in enumerate((c, g) for c in UP_WIDTHS for g in UP_GRIDS)},
+    "upsample_geo_bench_19_37": lambda: chk_upsample_geo(256, [(19, 19, 37, 37)], 32, seed=90),
+    "upsample_geo_bench_148_296": lambda: chk_upsample_geo(256, [(148, 148, 296, 296)], 32, (0, 16, 31), seed=91),
+    **{f"patch_gather_geo_{r[0]}x{r[1]}x{r[2]}_g{sum(r[3])}": (lambda r=r, i=i: chk_patch_gather_geo(*r, seed=i))
+       for i, r in enumerate(PG_ROWS)},
 }
 
 
