@@ -109,6 +109,11 @@ SIGNATURES = {
     "ada_pre_mask_nearest": (c_int32, [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_int32, c_int32, c_void_p]),
     "ada_post_minmax_normalize": (c_int32, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "ada_post_blend_seam": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p]),
+    "ada_pre_resize_linear_batch": (c_int32, [c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_int32, c_void_p]),
+    "ada_pre_image_nearest_batch": (c_int32, [c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_int32, c_int32, c_void_p]),
+    "ada_pre_mask_nearest_batch": (c_int32, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_int32, c_void_p]),
+    "ada_post_minmax_normalize_batch": (c_int32, [c_void_p, c_int32, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ada_post_blend_seam_batch": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p]),
     "ada_eval_sample": (c_int32, [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p,
                                   c_void_p, c_void_p]),
     "ada_op_attention": (c_int32, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p]),

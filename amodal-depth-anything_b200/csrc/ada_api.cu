@@ -2100,13 +2100,15 @@ int ada_op_layernorm(float* x, const void* delta_bf16, const void* delta2_bf16, 
   });
 }
 
-// ---- single-image pre/post-processing of infer.py (SURVEY.md section 8 row f2)
+// ---- pre/post-processing of infer.py (SURVEY.md section 8 row f2): the single-image entry points launch the batched
+// kernels with B = 1 and no descriptor table
 int ada_pre_image_nearest(const uint8_t* img_hwc, int32_t H0, int32_t W0, float* out_chw, int32_t H, int32_t W,
                           int32_t normalize, void* stream) {
   return guarded([&] {
     require_device();
     ADA_REQUIRE(img_hwc && out_chw && H0 > 0 && W0 > 0 && H > 0 && W > 0, "bad argument");
-    image_nearest_kernel<<<(H * W + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(img_hwc, H0, W0, out_chw, H, W, normalize);
+    image_nearest_kernel<<<dim3((H * W + 255) / 256, 1), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        img_hwc, nullptr, H0, W0, out_chw, H, W, normalize);
     ADA_CHECK_CUDA(cudaGetLastError());
   });
 }
@@ -2116,22 +2118,27 @@ int ada_pre_mask_nearest(const uint8_t* mask, int32_t H0, int32_t W0, float* mas
   return guarded([&] {
     require_device();
     ADA_REQUIRE(mask && (mask01 || guide) && H0 > 0 && W0 > 0 && H > 0 && W > 0, "bad argument");
-    mask_nearest_kernel<<<(H * W + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(mask, H0, W0, mask01, guide, H, W);
+    mask_nearest_kernel<<<dim3((H * W + 255) / 256, 1), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        mask, nullptr, H0, W0, mask01, guide, H, W);
     ADA_CHECK_CUDA(cudaGetLastError());
   });
+}
+
+static void launch_minmax_normalize(const float* depth, int B, long long n, float* base01, float* obs, void* scratch,
+                                    cudaStream_t st) {
+  uint32_t* mm = static_cast<uint32_t*>(scratch);
+  const int gx = static_cast<int>(std::min<long long>((n + 255) / 256, std::max(1, 148 * 8 / B)));
+  minmax_init_kernel<<<1, 256, 0, st>>>(mm, B);
+  minmax_kernel<<<dim3(gx, B), 256, 0, st>>>(depth, n, mm);
+  normalize_kernel<<<dim3(gx, B), 256, 0, st>>>(depth, n, mm, base01, obs);
+  ADA_CHECK_CUDA(cudaGetLastError());
 }
 
 int ada_post_minmax_normalize(const float* depth, int64_t n, float* base01, float* obs, void* scratch8, void* stream) {
   return guarded([&] {
     require_device();
     ADA_REQUIRE(depth && (base01 || obs) && scratch8 && n > 0, "bad argument");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    uint32_t* mm = static_cast<uint32_t*>(scratch8);
-    const int grid = static_cast<int>(std::min<long long>((n + 255) / 256, 148LL * 8));
-    minmax_init_kernel<<<1, 1, 0, st>>>(mm);
-    minmax_kernel<<<grid, 256, 0, st>>>(depth, n, mm);
-    normalize_kernel<<<grid, 256, 0, st>>>(depth, n, mm, base01, obs);
-    ADA_CHECK_CUDA(cudaGetLastError());
+    launch_minmax_normalize(depth, 1, n, base01, obs, scratch8, static_cast<cudaStream_t>(stream));
   });
 }
 
@@ -2141,7 +2148,72 @@ int ada_post_blend_seam(const float* raw01, const float* amodal, const float* ma
     require_device();
     ADA_REQUIRE(raw01 && amodal && mask01 && out && H > 1 && W > 1, "bad argument");
     ADA_REQUIRE(out != raw01 && out != amodal, "blend_seam is not in-place safe");
-    blend_seam_kernel<<<(H * W + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(raw01, amodal, mask01, out, H, W);
+    blend_seam_kernel<<<dim3((H * W + 255) / 256, 1), 256, 0, static_cast<cudaStream_t>(stream)>>>(raw01, amodal, mask01,
+                                                                                                   out, H, W);
+    ADA_CHECK_CUDA(cudaGetLastError());
+  });
+}
+
+static void require_batch(int B, int H, int W) {
+  ADA_REQUIRE(B > 0 && B <= 65535, "batch must be in [1, 65535]");
+  ADA_REQUIRE(H > 0 && W > 0 && static_cast<long long>(H) * W < (1LL << 31) / 3, "bad output size");
+}
+
+int ada_pre_resize_linear_batch(const uint8_t* src, const ada_img_desc* desc, int32_t B, uint8_t* out_hwc, int32_t H,
+                                int32_t W, void* stream) {
+  return guarded([&] {
+    require_device();
+    ADA_REQUIRE(src && desc && out_hwc, "bad argument");
+    require_batch(B, H, W);
+    resize_linear_kernel<<<dim3((H * W + 255) / 256, B), 256, 0, static_cast<cudaStream_t>(stream)>>>(src, desc, out_hwc,
+                                                                                                      H, W);
+    ADA_CHECK_CUDA(cudaGetLastError());
+  });
+}
+
+int ada_pre_image_nearest_batch(const uint8_t* src, const ada_img_desc* desc, int32_t B, float* out_chw, int32_t H,
+                                int32_t W, int32_t normalize, void* stream) {
+  return guarded([&] {
+    require_device();
+    ADA_REQUIRE(src && desc && out_chw, "bad argument");
+    require_batch(B, H, W);
+    image_nearest_kernel<<<dim3((H * W + 255) / 256, B), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        src, desc, 0, 0, out_chw, H, W, normalize);
+    ADA_CHECK_CUDA(cudaGetLastError());
+  });
+}
+
+int ada_pre_mask_nearest_batch(const uint8_t* src, const ada_img_desc* desc, int32_t B, float* mask01, float* guide,
+                               int32_t H, int32_t W, void* stream) {
+  return guarded([&] {
+    require_device();
+    ADA_REQUIRE(src && desc && (mask01 || guide), "bad argument");
+    require_batch(B, H, W);
+    mask_nearest_kernel<<<dim3((H * W + 255) / 256, B), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        src, desc, 0, 0, mask01, guide, H, W);
+    ADA_CHECK_CUDA(cudaGetLastError());
+  });
+}
+
+int ada_post_minmax_normalize_batch(const float* depth, int32_t B, int64_t n, float* base01, float* obs, void* scratch,
+                                    void* stream) {
+  return guarded([&] {
+    require_device();
+    ADA_REQUIRE(depth && (base01 || obs) && scratch && n > 0, "bad argument");
+    ADA_REQUIRE(B > 0 && B <= 65535, "batch must be in [1, 65535]");
+    launch_minmax_normalize(depth, B, n, base01, obs, scratch, static_cast<cudaStream_t>(stream));
+  });
+}
+
+int ada_post_blend_seam_batch(const float* raw01, const float* amodal, const float* mask01, float* out, int32_t B,
+                              int32_t H, int32_t W, void* stream) {
+  return guarded([&] {
+    require_device();
+    ADA_REQUIRE(raw01 && amodal && mask01 && out && H > 1 && W > 1, "bad argument");
+    ADA_REQUIRE(out != raw01 && out != amodal, "blend_seam is not in-place safe");
+    require_batch(B, H, W);
+    blend_seam_kernel<<<dim3((H * W + 255) / 256, B), 256, 0, static_cast<cudaStream_t>(stream)>>>(raw01, amodal, mask01,
+                                                                                                   out, H, W);
     ADA_CHECK_CUDA(cudaGetLastError());
   });
 }

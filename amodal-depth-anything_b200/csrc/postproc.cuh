@@ -1,53 +1,119 @@
 // Device-side pre/post-processing of the reference's single-image inference (infer.py:16-28, 72-103; SURVEY.md section 8
-// row f2). In the reference these steps bounce through the host (depth_raw.cpu() -> normalise -> .cuda(), pred.cpu() ->
-// numpy blend -> cv2.blur); here they are small bandwidth kernels on the forward's stream. All fp32, single image.
+// row f2). In the reference these steps bounce through the host (cv2.resize, depth_raw.cpu() -> normalise -> .cuda(),
+// pred.cpu() -> numpy blend -> cv2.blur); here they are small bandwidth kernels on the forward's stream. All fp32 except
+// the uint8 resize. Every kernel runs over a batch: image b is blockIdx.y. Images of different sizes are read from one
+// packed uint8 buffer through a device table of ada_img_desc rows; the single-image entry points launch the same kernels
+// with one image and no table.
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "../../include/amodal_b200.h"
+
 namespace ada {
+
+// Geometry of image blockIdx.y: its row of the descriptor table, or, without a table (the single-image entry points),
+// the one image at src of H0 x W0.
+__device__ __forceinline__ ada_img_desc image_desc(const ada_img_desc* __restrict__ table, int H0, int W0) {
+  if (table) return table[blockIdx.y];
+  return ada_img_desc{0, H0, W0};
+}
 
 // ATen nearest (F.interpolate default / torchvision Resize(NEAREST), infer.py:85-87,97-100): src = min(floor(dst * in/out), in-1)
 __device__ __forceinline__ int nearest_src(int dst, float scale, int in) {
   return min(static_cast<int>(floorf(static_cast<float>(dst) * scale)), in - 1);
 }
 
-// uint8 HWC image (cv2 order, infer.py:76) -> fp32 CHW in [0,1] at (H, W) by nearest sampling: rgb/255 then Resize(NEAREST)
-// (infer.py:84-86). normalize != 0 additionally applies (x - mean) / std with the ImageNet constants per channel index
-// (infer.py:18, the un-guided model's input). One thread per output pixel, 3 channels.
+// cv2.resize(img, (W, H)) with INTER_LINEAR on uint8 HWC, 3 channels (infer.py:17), bit-exact. Source coordinate and
+// 11-bit coefficients of output index d along an axis of `src` -> `dst` samples, as OpenCV computes them: the coordinate
+// in double rounded to float, the fraction in float, each coefficient rounded half to even on its own. Explicit _rn
+// intrinsics keep the compiler from contracting these into FMAs, which would round differently.
+__device__ __forceinline__ void linear_coeff(int d, int dst, int src, int& s, int& a0, int& a1) {
+  const double scale = __ddiv_rn(1.0, __ddiv_rn(static_cast<double>(dst), static_cast<double>(src)));
+  float f = __double2float_rn(__dadd_rn(__dmul_rn(__dadd_rn(static_cast<double>(d), 0.5), scale), -0.5));
+  const float fs = floorf(f);
+  s = static_cast<int>(fs);
+  f = __fsub_rn(f, fs);
+  a0 = __float2int_rn(__fmul_rn(__fsub_rn(1.0f, f), 2048.0f));
+  a1 = __float2int_rn(__fmul_rn(f, 2048.0f));
+}
+// One thread per output pixel of image blockIdx.y; out is [B, H, W, 3]. Along x the border resets the fraction; along y
+// it does not, only the two source rows are clamped (OpenCV's vertical pass clamps row pointers, not coefficients).
+// OpenCV takes its INTER_AREA fast path, (a + b + c + d + 2) >> 2, when the image is exactly 2H x 2W; this arithmetic
+// gives the same bits there (all four coefficients are 1024, so each vertical term is exactly a + b).
 __global__ void __launch_bounds__(256)
-image_nearest_kernel(const uint8_t* __restrict__ img, int H0, int W0, float* __restrict__ out, int H, int W, int normalize) {
+resize_linear_kernel(const uint8_t* __restrict__ src, const ada_img_desc* __restrict__ table, uint8_t* __restrict__ out,
+                     int H, int W) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= H * W) return;
   const int y = i / W, x = i - y * W;
+  const ada_img_desc g = table[blockIdx.y];
+  const int H0 = static_cast<int>(g.H0), W0 = static_cast<int>(g.W0);
+  const uint8_t* img = src + g.offset;
+  uint8_t* o = out + (static_cast<long long>(blockIdx.y) * H * W + i) * 3;
+  int sx, a0, a1, sy, b0, b1;
+  linear_coeff(x, W, W0, sx, a0, a1);
+  linear_coeff(y, H, H0, sy, b0, b1);
+  if (sx < 0 || sx >= W0 - 1) {
+    sx = sx < 0 ? 0 : W0 - 1;
+    a0 = 2048;
+    a1 = 0;
+  }
+  const int sx1 = min(sx + 1, W0 - 1);
+  const uint8_t* r0 = img + static_cast<long long>(min(max(sy, 0), H0 - 1)) * W0 * 3;
+  const uint8_t* r1 = img + static_cast<long long>(min(max(sy + 1, 0), H0 - 1)) * W0 * 3;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const int S0 = r0[sx * 3 + c] * a0 + r0[sx1 * 3 + c] * a1;
+    const int S1 = r1[sx * 3 + c] * a0 + r1[sx1 * 3 + c] * a1;
+    o[c] = static_cast<uint8_t>((((b0 * (S0 >> 4)) >> 16) + ((b1 * (S1 >> 4)) >> 16) + 2) >> 2);
+  }
+}
+
+// uint8 HWC image (cv2 order, infer.py:76) -> fp32 CHW in [0,1] at (H, W) by nearest sampling: rgb/255 then Resize(NEAREST)
+// (infer.py:84-86). normalize != 0 additionally applies (x - mean) / std with the ImageNet constants per channel index
+// (infer.py:18, the un-guided model's input). One thread per output pixel, 3 channels; out is [B, 3, H, W].
+__global__ void __launch_bounds__(256)
+image_nearest_kernel(const uint8_t* __restrict__ src, const ada_img_desc* __restrict__ table, int H0_, int W0_,
+                     float* __restrict__ out, int H, int W, int normalize) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= H * W) return;
+  const ada_img_desc g = image_desc(table, H0_, W0_);
+  const int H0 = static_cast<int>(g.H0), W0 = static_cast<int>(g.W0);
+  const int y = i / W, x = i - y * W;
   const int sy = nearest_src(y, static_cast<float>(H0) / static_cast<float>(H), H0);
   const int sx = nearest_src(x, static_cast<float>(W0) / static_cast<float>(W), W0);
-  const uint8_t* p = img + (static_cast<long long>(sy) * W0 + sx) * 3;
+  const uint8_t* p = src + g.offset + (static_cast<long long>(sy) * W0 + sx) * 3;
+  float* o = out + static_cast<long long>(blockIdx.y) * 3 * H * W;
   const float mean[3] = {0.485f, 0.456f, 0.406f}, sd[3] = {0.229f, 0.224f, 0.225f};
 #pragma unroll
   for (int c = 0; c < 3; ++c) {
     float v = static_cast<float>(p[c]) / 255.0f;
     if (normalize) v = __fdiv_rn(__fsub_rn(v, mean[c]), sd[c]);  // same two roundings as the tensor expression
-    out[static_cast<long long>(c) * H * W + i] = v;
+    o[static_cast<long long>(c) * H * W + i] = v;
   }
 }
 
 // uint8 mask (any non-zero = inside, infer.py:80-81) -> nearest resize -> mask01 (0/1, infer.py:87,100-101) and the
-// network guide mask01 * 2 - 1 (infer.py:91). Either output may be null.
+// network guide mask01 * 2 - 1 (infer.py:91), each [B, H, W]. Either output may be null.
 __global__ void __launch_bounds__(256)
-mask_nearest_kernel(const uint8_t* __restrict__ mask, int H0, int W0, float* __restrict__ mask01, float* __restrict__ guide,
-                    int H, int W) {
+mask_nearest_kernel(const uint8_t* __restrict__ src, const ada_img_desc* __restrict__ table, int H0_, int W0_,
+                    float* __restrict__ mask01, float* __restrict__ guide, int H, int W) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= H * W) return;
+  const ada_img_desc g = image_desc(table, H0_, W0_);
+  const int H0 = static_cast<int>(g.H0), W0 = static_cast<int>(g.W0);
   const int y = i / W, x = i - y * W;
   const int sy = nearest_src(y, static_cast<float>(H0) / static_cast<float>(H), H0);
   const int sx = nearest_src(x, static_cast<float>(W0) / static_cast<float>(W), W0);
-  const float m = mask[static_cast<long long>(sy) * W0 + sx] > 0 ? 1.0f : 0.0f;
-  if (mask01) mask01[i] = m;
-  if (guide) guide[i] = m * 2.0f - 1.0f;
+  const float m = src[g.offset + static_cast<long long>(sy) * W0 + sx] > 0 ? 1.0f : 0.0f;
+  const long long j = static_cast<long long>(blockIdx.y) * H * W + i;
+  if (mask01) mask01[j] = m;
+  if (guide) guide[j] = m * 2.0f - 1.0f;
 }
 
-// min / max of a fp32 map (infer.py:22). Order-preserving float <-> uint mapping so atomicMin/Max work for any sign.
+// min / max of each of B fp32 maps of n values (infer.py:22): mm[2b] / mm[2b+1] for map b = blockIdx.y.
+// Order-preserving float <-> uint mapping so atomicMin/Max work for any sign.
 __device__ __forceinline__ uint32_t f2ord(float f) {
   const uint32_t u = __float_as_uint(f);
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
@@ -55,12 +121,16 @@ __device__ __forceinline__ uint32_t f2ord(float f) {
 __device__ __forceinline__ float ord2f(uint32_t o) {
   return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
 }
-__global__ void minmax_init_kernel(uint32_t* mm) {
-  mm[0] = 0xffffffffu;  // min
-  mm[1] = 0u;           // max
+__global__ void minmax_init_kernel(uint32_t* mm, int B) {
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    mm[2 * b] = 0xffffffffu;  // min
+    mm[2 * b + 1] = 0u;       // max
+  }
 }
 __global__ void __launch_bounds__(256)
 minmax_kernel(const float* __restrict__ d, long long n, uint32_t* mm) {
+  d += static_cast<long long>(blockIdx.y) * n;
+  mm += 2 * blockIdx.y;
   uint32_t lo = 0xffffffffu, hi = 0u;
   for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
@@ -78,23 +148,25 @@ minmax_kernel(const float* __restrict__ d, long long n, uint32_t* mm) {
     atomicMax(mm + 1, hi);
   }
 }
-// base01 = (d - min) / (max - min) (infer.py:22); observation = base01 * 2 - 1 (infer.py:92). Either output may be null.
+// base01 = (d - min) / (max - min) (infer.py:22); observation = base01 * 2 - 1 (infer.py:92), per map. Either output may
+// be null. A constant map gives 0/0 = NaN, as the reference does.
 __global__ void __launch_bounds__(256)
 normalize_kernel(const float* __restrict__ d, long long n, const uint32_t* __restrict__ mm, float* __restrict__ base01,
                  float* __restrict__ obs) {
-  const float lo = ord2f(mm[0]), hi = ord2f(mm[1]);
+  const long long off = static_cast<long long>(blockIdx.y) * n;
+  const float lo = ord2f(mm[2 * blockIdx.y]), hi = ord2f(mm[2 * blockIdx.y + 1]);
   const float range = hi - lo;
   for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const float v = (d[i] - lo) / range;
-    if (base01) base01[i] = v;
-    if (obs) obs[i] = v * 2.0f - 1.0f;
+    const float v = (d[off + i] - lo) / range;
+    if (base01) base01[off + i] = v;
+    if (obs) obs[off + i] = v * 2.0f - 1.0f;
   }
 }
 
 // median_filter_blend (infer.py:30-44, filter_width 3): blended = mask ? amodal : raw; the seam = pixels whose 3x3
 // zero-padded mask sum is in (0, 9) is replaced by the 3x3 box mean of `blended` (cv2.blur: BORDER_REFLECT_101, row sums
-// then column sum, times 1/9 in fp32).
+// then column sum, times 1/9 in fp32). All maps [B, H, W]; map b = blockIdx.y.
 __device__ __forceinline__ int reflect101(int i, int n) {
   if (i < 0) return -i;
   if (i >= n) return 2 * n - 2 - i;
@@ -105,6 +177,10 @@ blend_seam_kernel(const float* __restrict__ raw, const float* __restrict__ amoda
                   float* __restrict__ out, int H, int W) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= H * W) return;
+  const long long off = static_cast<long long>(blockIdx.y) * H * W;
+  raw += off;
+  amodal += off;
+  mask01 += off;
   const int y = i / W, x = i - y * W;
   auto blended = [&](int yy, int xx) {
     const int j = yy * W + xx;
@@ -128,7 +204,7 @@ blend_seam_kernel(const float* __restrict__ raw, const float* __restrict__ amoda
     }
     v = ((rows[0] + rows[1]) + rows[2]) * (1.0f / 9.0f);
   }
-  out[i] = v;
+  out[off + i] = v;
 }
 
 }  // namespace ada

@@ -3,6 +3,7 @@ against the matching torch op; the model path (model.py) calls ada_forward direc
 from __future__ import annotations
 
 import ctypes
+import math
 
 import torch
 
@@ -212,6 +213,80 @@ def blend_seam(raw01, amodal, mask01):
     H, W = raw01.shape[-2:]
     out = torch.empty(H, W, dtype=torch.float32, device=raw01.device)
     _call(raw01, L.load().ada_post_blend_seam, _p(raw01.contiguous()), _p(amodal.contiguous()), _p(mask01.contiguous()), _p(out), H, W)
+    return out
+
+
+# ---- the same pre/post-processing over a batch (include/amodal_b200.h, ada_*_batch): images of any size packed into one
+#      uint8 device buffer, located by a descriptor table, int64 [B, 3] rows of {byte offset, H0, W0} (ada_img_desc)
+def pack_layout(shapes, start=0):
+    """Descriptor rows placing uint8 arrays of the given shapes ([H0, W0] or [H0, W0, C]) one after another from byte
+    `start`, each at a 16-byte boundary. Returns (rows, end byte)."""
+    rows, off = [], start
+    for shp in shapes:
+        off = (off + 15) // 16 * 16
+        rows.append((off, shp[0], shp[1]))
+        off += math.prod(shp)
+    return rows, off
+
+
+def _desc(src, desc):
+    assert src.dtype == torch.uint8 and src.is_contiguous()
+    assert desc.dtype == torch.int64 and desc.dim() == 2 and desc.shape[1] == 3 and desc.is_contiguous()
+    assert desc.device == src.device
+    return desc.shape[0]
+
+
+def _out(out, shape, dtype, device):
+    if out is None:
+        return torch.empty(shape, dtype=dtype, device=device)
+    assert tuple(out.shape) == tuple(shape) and out.dtype == dtype and out.is_contiguous()
+    return out
+
+
+def resize_linear_batch(src_u8, desc, H=518, W=518, out=None):
+    """cv2.resize(img, (W, H)) (INTER_LINEAR, infer.py:17) of each 3-channel image of the packed buffer, bit-exact ->
+    uint8 [B,H,W,3]."""
+    B = _desc(src_u8, desc)
+    out = _out(out, (B, H, W, 3), torch.uint8, src_u8.device)
+    _call(src_u8, L.load().ada_pre_resize_linear_batch, _p(src_u8), _p(desc), B, _p(out), H, W)
+    return out
+
+
+def image_nearest_batch(src_u8, desc, H=518, W=518, normalize=False, out=None):
+    """image_nearest of each 3-channel image of the packed buffer -> fp32 [B,3,H,W]."""
+    B = _desc(src_u8, desc)
+    out = _out(out, (B, 3, H, W), torch.float32, src_u8.device)
+    _call(src_u8, L.load().ada_pre_image_nearest_batch, _p(src_u8), _p(desc), B, _p(out), H, W, int(normalize))
+    return out
+
+
+def mask_nearest_batch(src_u8, desc, H=518, W=518, mask01=None, guide=None):
+    """mask_nearest of each mask of the packed buffer -> (mask01 [B,1,H,W], guide [B,1,H,W])."""
+    B = _desc(src_u8, desc)
+    mask01 = _out(mask01, (B, 1, H, W), torch.float32, src_u8.device)
+    guide = _out(guide, (B, 1, H, W), torch.float32, src_u8.device)
+    _call(src_u8, L.load().ada_pre_mask_nearest_batch, _p(src_u8), _p(desc), B, _p(mask01), _p(guide), H, W)
+    return mask01, guide
+
+
+def minmax_normalize_batch(depth):
+    """minmax_normalize of each depth[b] (min and max per map) -> (base01, observation), depth's shape."""
+    d = depth.contiguous()
+    B = d.shape[0]
+    base, obs = torch.empty_like(d), torch.empty_like(d)
+    scratch = torch.empty(2 * B, dtype=torch.int32, device=d.device)
+    _call(d, L.load().ada_post_minmax_normalize_batch, _p(d), B, d.numel() // B, _p(base), _p(obs), _p(scratch))
+    return base, obs
+
+
+def blend_seam_batch(raw01, amodal, mask01):
+    """blend_seam of each map: raw01 / amodal / mask01 [B,H,W] (or [B,1,H,W]) -> [B,H,W]."""
+    B = raw01.shape[0]
+    H, W = raw01.shape[-2:]
+    raw01, amodal, mask01 = raw01.contiguous(), amodal.contiguous(), mask01.contiguous()
+    assert raw01.numel() == amodal.numel() == mask01.numel() == B * H * W
+    out = torch.empty(B, H, W, dtype=torch.float32, device=raw01.device)
+    _call(raw01, L.load().ada_post_blend_seam_batch, _p(raw01), _p(amodal), _p(mask01), _p(out), B, H, W)
     return out
 
 

@@ -170,6 +170,33 @@ int ada_post_minmax_normalize(const float* depth, int64_t n, float* base01, floa
  * (3x3 zero-padded mask sum in (0,9)) replaced by the 3x3 box mean of the blended map (cv2.blur, BORDER_REFLECT_101). */
 int ada_post_blend_seam(const float* raw01, const float* amodal, const float* mask01, float* out, int32_t H, int32_t W,
                         void* stream);
+/* ---- the same pre/post-processing over a batch of B images (B <= 65535), each image's result bit-equal to the
+ * single-image entry point's on that image. Images of different sizes live in one packed uint8 device buffer `src`;
+ * desc (device, B rows) gives each one's byte offset into it and its size. The rows are read by the kernels, not
+ * checked on the host: every image must lie inside `src`. Outputs are dense batches: image b at b * (its per-image
+ * size). */
+typedef struct ada_img_desc {
+  int64_t offset; /* bytes from src to the image's first element */
+  int64_t H0, W0; /* its rows and columns (> 0) */
+} ada_img_desc;
+/* cv2.resize(img, (W, H)) with the default INTER_LINEAR (infer.py:17), bit-exact: uint8 HWC 3-channel images ->
+ * out [B,H,W,3] uint8. OpenCV's fixed-point arithmetic (11-bit coefficients); it also equals OpenCV's INTER_AREA path,
+ * which cv2 takes when the image is exactly 2H x 2W. An image already H x W comes out unchanged. */
+int ada_pre_resize_linear_batch(const uint8_t* src, const ada_img_desc* desc, int32_t B, uint8_t* out_hwc, int32_t H,
+                                int32_t W, void* stream);
+/* ada_pre_image_nearest per image (3-channel rows of desc) -> out [B,3,H,W]. */
+int ada_pre_image_nearest_batch(const uint8_t* src, const ada_img_desc* desc, int32_t B, float* out_chw, int32_t H,
+                                int32_t W, int32_t normalize, void* stream);
+/* ada_pre_mask_nearest per image (1-channel rows of desc) -> mask01 / guide [B,H,W]; either may be NULL. */
+int ada_pre_mask_nearest_batch(const uint8_t* src, const ada_img_desc* desc, int32_t B, float* mask01, float* guide,
+                               int32_t H, int32_t W, void* stream);
+/* ada_post_minmax_normalize on each of B maps of n values (depth [B,n]), min and max per map; scratch = 8*B bytes of
+ * device memory. */
+int ada_post_minmax_normalize_batch(const float* depth, int32_t B, int64_t n, float* base01, float* obs, void* scratch,
+                                    void* stream);
+/* ada_post_blend_seam on each of B maps: raw01, amodal, mask01, out [B,H,W]. */
+int ada_post_blend_seam_batch(const float* raw01, const float* amodal, const float* mask01, float* out, int32_t B,
+                              int32_t H, int32_t W, void* stream);
 /* ---- per-sample evaluation post-ops of the validation loop on the device (SURVEY.md section 8 row f3;
  * discriminative_trainer.py:542-613). pred [h,w] is resized to the ground-truth size (H,W) by nearest sampling (:542),
  * aligned to depth_obs over visible_mask by least squares (src/util/alignment.py:7-54) and scored against depth_gt + 1e-5
