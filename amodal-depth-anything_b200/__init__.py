@@ -5,7 +5,8 @@ The directory name carries a hyphen (it mirrors the reference repo name); import
 (the shim of that name at the repo root loads this package).
 """
 from . import _lib  # noqa: F401  (ctypes binding; loading the .so is deferred to first use)
+from .evaluate import AmodalEvaluator  # noqa: F401
 from .infer import AmodalInference  # noqa: F401
 from .model import GUIDE_CHANNELS, MODEL_CONFIGS, AmodalDAv2, DepthAnythingV2, get_model  # noqa: F401
 
-__all__ = ["AmodalDAv2", "DepthAnythingV2", "AmodalInference", "get_model", "MODEL_CONFIGS", "GUIDE_CHANNELS", "_lib"]
+__all__ = ["AmodalDAv2", "DepthAnythingV2", "AmodalInference", "AmodalEvaluator", "get_model", "MODEL_CONFIGS", "GUIDE_CHANNELS", "_lib"]

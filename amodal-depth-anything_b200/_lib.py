@@ -116,6 +116,8 @@ SIGNATURES = {
     "ada_post_blend_seam_batch": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p]),
     "ada_eval_sample": (c_int32, [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p,
                                   c_void_p, c_void_p]),
+    "ada_eval_batch": (c_int32, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p]),
+    "ada_eval_accumulate": (c_int32, [c_void_p, c_int32, c_void_p, c_int32, c_void_p, c_void_p]),
     "ada_op_attention": (c_int32, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p]),
     "ada_op_channel_ln_relu": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_float, c_void_p]),
     "ada_op_upsample": (c_int32, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p]),

@@ -2218,7 +2218,14 @@ int ada_post_blend_seam_batch(const float* raw01, const float* amodal, const flo
   });
 }
 
-// ---- per-sample evaluation post-ops of the validation loop (SURVEY.md section 8 row f3)
+// ---- per-sample evaluation post-ops of the validation loop (SURVEY.md section 8 row f3): ada_eval_sample launches the
+// batched kernel with B = 1 and no descriptor table
+static void launch_eval(const float* pred, const uint8_t* src, const ada_eval_desc* desc, const EvalSample& one, int B,
+                        double* out, cudaStream_t st) {
+  eval_batch_kernel<<<dim3(kEvalCluster, B), kEvalThreads, 0, st>>>(pred, src, desc, one, out);
+  ADA_CHECK_CUDA(cudaGetLastError());
+}
+
 int ada_eval_sample(const float* pred, int32_t h, int32_t w, const float* depth_gt, const float* depth_obs,
                     const uint8_t* visible_mask, const uint8_t* object_mask, int32_t H, int32_t W, double* out24,
                     double* scratch26, void* stream) {
@@ -2226,13 +2233,27 @@ int ada_eval_sample(const float* pred, int32_t h, int32_t w, const float* depth_
     require_device();
     ADA_REQUIRE(pred && depth_gt && depth_obs && visible_mask && object_mask && out24 && scratch26, "bad argument");
     ADA_REQUIRE(h > 0 && w > 0 && H > 0 && W > 0 && static_cast<long long>(H) * W < (1LL << 31), "bad size");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    EvalArgs a{pred, h, w, depth_gt, depth_obs, visible_mask, object_mask, H, W, scratch26, out24};
-    ADA_CHECK_CUDA(cudaMemsetAsync(scratch26, 0, sizeof(double) * kEvalScratch, st));
-    const int grid = static_cast<int>(std::min<long long>((static_cast<long long>(H) * W + 255) / 256, 148LL * 4));
-    eval_align_sums_kernel<<<grid, 256, 0, st>>>(a);
-    eval_metric_sums_kernel<<<grid, 256, 0, st>>>(a);
-    eval_finalize_kernel<<<1, 1, 0, st>>>(a);
+    const EvalSample one{pred, h, w, depth_gt, depth_obs, visible_mask, object_mask, H, W};
+    launch_eval(nullptr, nullptr, nullptr, one, 1, out24, static_cast<cudaStream_t>(stream));
+  });
+}
+
+int ada_eval_batch(const float* pred, const uint8_t* src, const ada_eval_desc* desc, int32_t B, double* out, void* stream) {
+  return guarded([&] {
+    require_device();
+    ADA_REQUIRE(pred && src && desc && out, "bad argument");
+    ADA_REQUIRE(B > 0 && B <= 65535, "batch must be in [1, 65535]");
+    launch_eval(pred, src, desc, EvalSample{}, B, out, static_cast<cudaStream_t>(stream));
+  });
+}
+
+int ada_eval_accumulate(const double* rows, int32_t B, const int32_t* bucket, int32_t n_buckets, double* acc, void* stream) {
+  return guarded([&] {
+    require_device();
+    ADA_REQUIRE(rows && acc, "bad argument");
+    ADA_REQUIRE(B > 0 && B <= 65535, "batch must be in [1, 65535]");
+    ADA_REQUIRE(n_buckets >= 0 && n_buckets <= 65535, "n_buckets must be in [0, 65535]");
+    eval_accumulate_kernel<<<1, 256, 0, static_cast<cudaStream_t>(stream)>>>(rows, B, bucket, n_buckets, acc);
     ADA_CHECK_CUDA(cudaGetLastError());
   });
 }

@@ -386,6 +386,11 @@ __device__ __forceinline__ uint32_t mapa_shared(uint32_t addr, uint32_t rank) {
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
   return r;
 }
+__device__ __forceinline__ double ld_shared_cluster_f64(uint32_t cluster_addr) {
+  double v;
+  asm volatile("ld.shared::cluster.f64 %0, [%1];" : "=d"(v) : "r"(cluster_addr) : "memory");
+  return v;
+}
 __device__ __forceinline__ void mbar_expect_tx_cluster(uint32_t cluster_bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cluster.b64 _, [%0], %1;" ::"r"(cluster_bar), "r"(bytes) : "memory");
 }

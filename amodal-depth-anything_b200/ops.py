@@ -309,6 +309,31 @@ def eval_sample(pred, depth_gt, depth_obs, visible_mask, object_mask):
     return out
 
 
+def eval_batch(pred, src_u8, desc, out=None):
+    """ada_eval_batch: the eval_sample post-ops of B samples of any sizes in one launch. pred: fp32 device tensor holding
+    every sample's [h, w] prediction; src_u8: uint8 device buffer holding their ground-truth maps; desc: int64 [B, 9]
+    device rows of ada_eval_desc (element offset into pred, byte offsets of depth_gt, depth_obs, visible, object into src,
+    then h, w, H, W). Returns [B, 24] float64 (row b bit-equal to eval_sample on sample b); no host synchronisation."""
+    assert pred.dtype == torch.float32 and pred.is_contiguous() and src_u8.dtype == torch.uint8 and src_u8.is_contiguous()
+    assert desc.dtype == torch.int64 and desc.dim() == 2 and desc.shape[1] == 9 and desc.is_contiguous()
+    assert pred.device == src_u8.device == desc.device
+    B = desc.shape[0]
+    out = _out(out, (B, 24), torch.float64, pred.device)
+    _call(pred, L.load().ada_eval_batch, _p(pred), _p(src_u8), _p(desc), B, _p(out))
+    return out
+
+
+def eval_accumulate(rows, bucket, n_buckets, acc):
+    """ada_eval_accumulate: acc [(n_buckets + 1), 22] float64 (row 0 overall, 1 + k bucket k: n_used, n_skipped, 20 metric
+    sums) += the [B, 24] rows, in row order; bucket: int32 [B] device labels or None (overall only)."""
+    assert rows.dtype == torch.float64 and rows.dim() == 2 and rows.shape[1] == 24 and rows.is_contiguous()
+    assert acc.dtype == torch.float64 and acc.numel() == (n_buckets + 1) * 22 and acc.is_contiguous()
+    if bucket is not None:
+        assert bucket.dtype == torch.int32 and bucket.numel() == rows.shape[0] and bucket.is_contiguous()
+    _call(rows, L.load().ada_eval_accumulate, _p(rows), rows.shape[0], _p(bucket), n_buckets, _p(acc))
+    return acc
+
+
 def eval_sample_dict(out24):
     """One host read of the 24 numbers -> {'scale', 'shift', 'pred': {metric: value}, 'aligned': {...}}."""
     v = out24.cpu().tolist()

@@ -203,10 +203,31 @@ int ada_post_blend_seam_batch(const float* raw01, const float* amodal, const flo
  * over object_mask with the ten metrics of src/util/metric.py:37-161, for the raw and the aligned prediction (:584-613).
  * out24 (device doubles): [0] scale, [1] shift, [2..11] metrics of pred, [12..21] metrics of the aligned prediction in the
  * order abs_relative_difference, squared_relative_difference, rmse_linear, rmse_log, log10, delta1_acc, delta2_acc,
- * delta3_acc, i_rmse, silog_rmse; [22] visible pixels, [23] object pixels. scratch26: 26 device doubles. Masks: uint8. */
+ * delta3_acc, i_rmse, silog_rmse; [22] visible pixels, [23] object pixels. Masks: uint8. scratch26 (26 device doubles) is
+ * checked for NULL but no longer written. Runs ada_eval_batch's kernel on one sample: the row is bit-equal to that
+ * sample's row in any batch, and the same on every run. */
 int ada_eval_sample(const float* pred, int32_t h, int32_t w, const float* depth_gt, const float* depth_obs,
                     const uint8_t* visible_mask, const uint8_t* object_mask, int32_t H, int32_t W, double* out24,
                     double* scratch26, void* stream);
+/* ada_eval_sample over a batch of B samples (B <= 65535) whose predictions and ground truths each have their own size.
+ * desc (device, B rows) locates sample b: its [h,w] prediction at pred + desc[b].pred (elements) and its four [H,W] maps
+ * at byte offsets from src (fp32 depth_gt, fp32 depth_obs, uint8 visible and object masks). The rows are read by the
+ * kernel, not checked on the host: every map must lie inside its buffer, fp32 maps 4-byte aligned, H*W < 2^31.
+ * out: [B,24] device doubles, row b in the out24 layout. Deterministic, no atomics: row b is bit-equal to ada_eval_sample
+ * on sample b, whatever the batch and on every run. */
+typedef struct ada_eval_desc {
+  int64_t pred;                        /* element offset of the sample's [h,w] prediction from `pred` */
+  int64_t gt, obs, visible, object;    /* byte offsets from `src` (fp32, fp32, uint8, uint8 maps of [H,W]) */
+  int64_t h, w, H, W;
+} ada_eval_desc;
+int ada_eval_batch(const float* pred, const uint8_t* src, const ada_eval_desc* desc, int32_t B, double* out, void* stream);
+/* Dataset means of the validation loop: adds the B rows [B,24] (ada_eval_batch's out) into acc, (n_buckets + 1) x 22 device
+ * doubles. Row 0 of acc is "overall", row 1 + k is bucket k; each holds n_used, n_skipped and the sums of the 20 metric
+ * values [2..21] of the rows it took. A row with a NaN among its 20 metric values is counted in n_skipped and left out of
+ * the sums (discriminative_trainer.py:596-597). bucket (device int32 [B], or NULL for "overall" only) labels the rows; a
+ * label outside [0, n_buckets) counts in "overall" only. Rows are added in order, so acc is the same bits however the
+ * samples are split into calls. 1 <= B <= 65535, 0 <= n_buckets <= 65535. */
+int ada_eval_accumulate(const double* rows, int32_t B, const int32_t* bucket, int32_t n_buckets, double* acc, void* stream);
 /* qkv bf16 [B,N,3,heads,64] -> out bf16 [B,N,heads*64] (attention.py:49-62). impl: -1 = the kernel ada_forward would pick for
  * this shape, 0 = attention.cuh (one 128-query tile per CTA), 1 = attention2.cuh (persistent, 256 queries per work unit). */
 int ada_op_attention(const void* qkv_bf16, void* out_bf16, int32_t B, int32_t N, int32_t heads, int32_t impl, void* stream);
