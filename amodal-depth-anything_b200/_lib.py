@@ -114,6 +114,8 @@ SIGNATURES = {
     "ada_pre_mask_nearest_batch": (c_int32, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_int32, c_void_p]),
     "ada_post_minmax_normalize_batch": (c_int32, [c_void_p, c_int32, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "ada_post_blend_seam_batch": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p]),
+    "ada_pre_resize_cubic_normalize_batch": (c_int32, [c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_int32, c_void_p]),
+    "ada_post_upsample_restore_batch": (c_int32, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
     "ada_eval_sample": (c_int32, [c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p,
                                   c_void_p, c_void_p]),
     "ada_eval_batch": (c_int32, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p]),

@@ -2218,6 +2218,32 @@ int ada_post_blend_seam_batch(const float* raw01, const float* amodal, const flo
   });
 }
 
+// ---- DepthAnythingV2.infer_image's pre/post-processing over a batch
+int ada_pre_resize_cubic_normalize_batch(const uint8_t* src, const ada_img_desc* desc, int32_t B, float* out_chw,
+                                         int32_t H, int32_t W, void* stream) {
+  return guarded([&] {
+    require_device();
+    ADA_REQUIRE(src && desc && out_chw, "bad argument");
+    require_batch(B, H, W);
+    resize_cubic_normalize_kernel<<<dim3((H * W + 255) / 256, B), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        src, desc, out_chw, H, W);
+    ADA_CHECK_CUDA(cudaGetLastError());
+  });
+}
+
+int ada_post_upsample_restore_batch(const float* depth, int32_t B, int32_t H, int32_t W, const ada_img_desc* out_desc,
+                                    float* out, void* stream) {
+  return guarded([&] {
+    require_device();
+    ADA_REQUIRE(depth && out_desc && out, "bad argument");
+    require_batch(B, H, W);
+    // the output sizes are on the device: a fixed grid of ~8 blocks per SM over the batch, striding over each image
+    const int gx = std::max(1, 148 * 8 / B);
+    upsample_restore_kernel<<<dim3(gx, B), 256, 0, static_cast<cudaStream_t>(stream)>>>(depth, H, W, out_desc, out);
+    ADA_CHECK_CUDA(cudaGetLastError());
+  });
+}
+
 // ---- per-sample evaluation post-ops of the validation loop (SURVEY.md section 8 row f3): ada_eval_sample launches the
 // batched kernel with B = 1 and no descriptor table
 static void launch_eval(const float* pred, const uint8_t* src, const ada_eval_desc* desc, const EvalSample& one, int B,

@@ -70,6 +70,65 @@ resize_linear_kernel(const uint8_t* __restrict__ src, const ada_img_desc* __rest
   }
 }
 
+// DepthAnythingV2.image2tensor (depth_anything_v2_raw/dpt.py:186-222), bit-exact: cvtColor(BGR -> RGB) / 255.0, then
+// cv2.resize(..., INTER_CUBIC) of that float64 image, then (x - mean) / std in float64, then astype(float32). OpenCV's
+// float64 cubic path computes the source coordinate as linear_coeff does, the four coefficients in float (A = -0.75, each
+// operation rounded on its own, the last one 1 - c0 - c1 - c2) and every sum in double, left to right, with the float
+// coefficients widened. Out-of-range source columns and rows are clamped (replicated), never reflected.
+__device__ __forceinline__ void cubic_coeff(int d, int dst, int src, int& s, float c[4]) {
+  const double scale = __ddiv_rn(1.0, __ddiv_rn(static_cast<double>(dst), static_cast<double>(src)));
+  float f = __double2float_rn(__dadd_rn(__dmul_rn(__dadd_rn(static_cast<double>(d), 0.5), scale), -0.5));
+  const float fs = floorf(f);
+  s = static_cast<int>(fs);
+  f = __fsub_rn(f, fs);
+  constexpr float A = -0.75f;
+  const float f1 = __fadd_rn(f, 1.0f), g = __fsub_rn(1.0f, f);
+  c[0] = __fsub_rn(__fmul_rn(__fadd_rn(__fmul_rn(__fsub_rn(__fmul_rn(A, f1), 5.0f * A), f1), 8.0f * A), f1), 4.0f * A);
+  c[1] = __fadd_rn(__fmul_rn(__fmul_rn(__fsub_rn(__fmul_rn(A + 2.0f, f), A + 3.0f), f), f), 1.0f);
+  c[2] = __fadd_rn(__fmul_rn(__fmul_rn(__fsub_rn(__fmul_rn(A + 2.0f, g), A + 3.0f), g), g), 1.0f);
+  c[3] = __fsub_rn(__fsub_rn(__fsub_rn(1.0f, c[0]), c[1]), c[2]);
+}
+// One thread per output pixel of image blockIdx.y (source geometry from its ada_img_desc row); out is [B, 3, H, W], the
+// ImageNet-normalised input DepthAnythingV2.forward expects. u / 255.0 comes from a per-block table of the 256 doubles.
+__global__ void __launch_bounds__(256)
+resize_cubic_normalize_kernel(const uint8_t* __restrict__ src, const ada_img_desc* __restrict__ table,
+                              float* __restrict__ out, int H, int W) {
+  __shared__ double unit[256];
+  unit[threadIdx.x] = __ddiv_rn(static_cast<double>(threadIdx.x), 255.0);
+  __syncthreads();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= H * W) return;
+  const int y = i / W, x = i - y * W;
+  const ada_img_desc g = table[blockIdx.y];
+  const int H0 = static_cast<int>(g.H0), W0 = static_cast<int>(g.W0);
+  const uint8_t* img = src + g.offset;
+  int sx, sy;
+  float cx[4], cy[4];
+  cubic_coeff(x, W, W0, sx, cx);
+  cubic_coeff(y, H, H0, sy, cy);
+  int col[4];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) col[k] = min(max(sx - 1 + k, 0), W0 - 1) * 3;
+  double v[3];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const uint8_t* r = img + static_cast<long long>(min(max(sy - 1 + k, 0), H0 - 1)) * W0 * 3;
+    const double wy = static_cast<double>(cy[k]);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {   // output channel c reads source channel 2 - c (BGR -> RGB)
+      double h = __dmul_rn(unit[r[col[0] + 2 - c]], static_cast<double>(cx[0]));
+#pragma unroll
+      for (int j = 1; j < 4; ++j) h = __dadd_rn(h, __dmul_rn(unit[r[col[j] + 2 - c]], static_cast<double>(cx[j])));
+      v[c] = k == 0 ? __dmul_rn(h, wy) : __dadd_rn(v[c], __dmul_rn(h, wy));
+    }
+  }
+  const double mean[3] = {0.485, 0.456, 0.406}, sd[3] = {0.229, 0.224, 0.225};
+  float* o = out + static_cast<long long>(blockIdx.y) * 3 * H * W + i;
+#pragma unroll
+  for (int c = 0; c < 3; ++c)
+    o[static_cast<long long>(c) * H * W] = __double2float_rn(__ddiv_rn(__dsub_rn(v[c], mean[c]), sd[c]));
+}
+
 // uint8 HWC image (cv2 order, infer.py:76) -> fp32 CHW in [0,1] at (H, W) by nearest sampling: rgb/255 then Resize(NEAREST)
 // (infer.py:84-86). normalize != 0 additionally applies (x - mean) / std with the ImageNet constants per channel index
 // (infer.py:18, the un-guided model's input). One thread per output pixel, 3 channels; out is [B, 3, H, W].
@@ -205,6 +264,42 @@ blend_seam_kernel(const float* __restrict__ raw, const float* __restrict__ amoda
     v = ((rows[0] + rows[1]) + rows[2]) * (1.0f / 9.0f);
   }
   out[off + i] = v;
+}
+
+// F.interpolate(depth[:, None], (h, w), mode="bilinear", align_corners=True) of DepthAnythingV2.infer_image
+// (depth_anything_v2_raw/dpt.py:186-222), with ATen's index math: scale (in - 1) / (out - 1) in fp32 (0 when out == 1),
+// src = scale * dst, i1 = i0 + (i0 < in - 1), lambda = src - i0. Every product and sum is rounded on its own. Map b =
+// blockIdx.y of depth [B, H, W] goes to its own (h, w) = (H0, W0) of its ada_img_desc row, at that row's byte offset
+// from out. The output sizes live on the device, so the threads of an image stride over its pixels.
+__device__ __forceinline__ void restore_coord(int d, int out, int in, int& i0, int& i1, float& l0, float& l1) {
+  const float scale = out > 1 ? __fdiv_rn(static_cast<float>(in - 1), static_cast<float>(out - 1)) : 0.0f;
+  const float s = __fmul_rn(scale, static_cast<float>(d));
+  i0 = static_cast<int>(s);
+  i1 = i0 + (i0 < in - 1 ? 1 : 0);
+  l1 = __fsub_rn(s, static_cast<float>(i0));
+  l0 = __fsub_rn(1.0f, l1);
+}
+__global__ void __launch_bounds__(256)
+upsample_restore_kernel(const float* __restrict__ depth, int H, int W, const ada_img_desc* __restrict__ table,
+                        float* __restrict__ out) {
+  const ada_img_desc g = table[blockIdx.y];
+  const int h = static_cast<int>(g.H0), w = static_cast<int>(g.W0);
+  const float* d = depth + static_cast<long long>(blockIdx.y) * H * W;
+  float* o = reinterpret_cast<float*>(reinterpret_cast<char*>(out) + g.offset);
+  const long long n = static_cast<long long>(h) * w;
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const int y = static_cast<int>(i / w), x = static_cast<int>(i - static_cast<long long>(y) * w);
+    int y0, y1, x0, x1;
+    float h0, h1, w0, w1;
+    restore_coord(y, h, H, y0, y1, h0, h1);
+    restore_coord(x, w, W, x0, x1, w0, w1);
+    const float* r0 = d + static_cast<long long>(y0) * W;
+    const float* r1 = d + static_cast<long long>(y1) * W;
+    const float top = __fadd_rn(__fmul_rn(w0, r0[x0]), __fmul_rn(w1, r0[x1]));
+    const float bot = __fadd_rn(__fmul_rn(w0, r1[x0]), __fmul_rn(w1, r1[x1]));
+    o[i] = __fadd_rn(__fmul_rn(h0, top), __fmul_rn(h1, bot));
+  }
 }
 
 }  // namespace ada

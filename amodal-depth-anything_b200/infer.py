@@ -23,9 +23,7 @@ class AmodalInference:
         self.model = depth_amodal_model.set_graph(cuda_graph)
         self.size = size
         self.device = next(depth_amodal_model.parameters()).device
-        self._pinned = None      # reused host staging of batch(): packed images + masks, and the descriptor table
-        self._pinned_desc = None
-        self._uploaded = None    # event after the last upload from the staging buffers (they are rewritten after it)
+        self._staging = ops.Staging(self.device)   # reused host staging of batch(): packed images + masks, descriptors
 
     def _upload_u8(self, a: np.ndarray) -> torch.Tensor:
         t = torch.from_numpy(np.ascontiguousarray(a))
@@ -80,24 +78,13 @@ class AmodalInference:
         rows_img, end = ops.pack_layout([a.shape for a in imgs])
         rows_mask, end = ops.pack_layout([m.shape for m in ms], end)
         rows = rows_img + rows_mask + [(b * S * S * 3, S, S) for b in range(B)]
-        if self._uploaded is not None:
-            self._uploaded.synchronize()         # the previous upload may still read the staging buffers
-        if self._pinned is None or self._pinned.numel() < end:
-            self._pinned = torch.empty(end, dtype=torch.uint8, pin_memory=True)
-        if self._pinned_desc is None or self._pinned_desc.shape[0] < len(rows):
-            self._pinned_desc = torch.empty(len(rows), 3, dtype=torch.int64, pin_memory=True)
-        host = self._pinned.numpy()
-        for (o, _, _), a in zip(rows_img, imgs):
-            np.copyto(host[o:o + a.size].reshape(a.shape), a)
-        for (o, _, _), m in zip(rows_mask, ms):
-            np.greater(m, 0, out=host[o:o + m.size].reshape(m.shape).view(np.bool_))   # as __call__ thresholds
-        self._pinned_desc.numpy()[:len(rows)] = rows
-        data = torch.empty(end, dtype=torch.uint8, device=self.device)
-        desc = torch.empty(len(rows), 3, dtype=torch.int64, device=self.device)
-        data.copy_(self._pinned[:end], non_blocking=True)
-        desc.copy_(self._pinned_desc[:len(rows)], non_blocking=True)
-        self._uploaded = torch.cuda.Event()
-        self._uploaded.record()
+
+        def fill(host):
+            for (o, _, _), a in zip(rows_img, imgs):
+                np.copyto(host[o:o + a.size].reshape(a.shape), a)
+            for (o, _, _), m in zip(rows_mask, ms):
+                np.greater(m, 0, out=host[o:o + m.size].reshape(m.shape).view(np.bool_))   # as __call__ thresholds
+        data, desc = self._staging.upload(end, rows, fill)
         return data, desc[:B], desc[B:2 * B], desc[2 * B:]
 
     def _batch(self, images, masks):

@@ -14,12 +14,14 @@ from __future__ import annotations
 import ctypes
 import math
 
+import numpy as np
 import torch
 import torch.nn as nn
 from huggingface_hub import PyTorchModelHubMixin
 from huggingface_hub.constants import SAFETENSORS_SINGLE_FILE
 
 from . import _lib as L
+from . import ops
 
 # dav2.py:31-34 (+ vitg), dpt.py:213-218, dinov2.py:366-427, swiglu_ffn.py:57
 MODEL_CONFIGS = {
@@ -171,6 +173,7 @@ class _NativeModel(nn.Module):
         state["_handle"] = None
         state["_handle_device"] = None
         state["_dirty"] = True
+        state.pop("_staging", None)   # DepthAnythingV2.infer_images' pinned buffers and event
         return state
 
     def _ensure_handle(self, device):
@@ -391,6 +394,56 @@ class DepthAnythingV2(_NativeModel):
         depth = self.forward(image)
         depth = torch.nn.functional.interpolate(depth[:, None], (h, w), mode="bilinear", align_corners=True)[0, 0]
         return depth.cpu().numpy()
+
+    @staticmethod
+    def _chunks(shapes, input_size, max_batch):
+        """The batches infer_images runs: [(H, W, [image indices])], images grouped by the network input size
+        _input_size picks for them, groups in order of first appearance, each cut into chunks of at most max_batch."""
+        groups = {}
+        for i, (h, w) in enumerate(shapes):
+            groups.setdefault(DepthAnythingV2._input_size(h, w, input_size), []).append(i)
+        return [(H, W, idx[k:k + max_batch]) for (H, W), idx in groups.items() for k in range(0, len(idx), max_batch)]
+
+    @torch.no_grad()
+    def infer_images(self, raw_images, input_size=518, max_batch=32):
+        """infer_image over a list, on the device: raw_images[i] is a uint8 BGR [h_i, w_i, 3] image (as cv2.imread returns
+        it); returns a list of fp32 device tensors [h_i, w_i] in input order, views into one packed buffer. Image i is
+        infer_image(raw_images[i], input_size) without the host read (call .cpu() on the results you need): the resize of
+        image2tensor (cv2's float64 INTER_CUBIC and the ImageNet normalise, bit-exact), the forward and the restore to
+        (h_i, w_i) all run as kernels on the current stream, and each image's result is bit-equal in any batch.
+
+        Images are grouped by the network input size _input_size picks for them; the groups run in order of first
+        appearance, each in chunks of at most max_batch images. The forward re-plans its workspace whenever (B, H, W)
+        changes (a drain of the stream, and a larger arena when the new shape needs one), so a call re-plans at most once
+        per distinct (B, H, W) of its chunks. Each chunk is one upload of the packed images and one of its descriptors.
+
+        Unlike infer_image, which also passes float images through cv2, only uint8 [h, w, 3] images are accepted: anything
+        else raises ValueError before any upload."""
+        if max_batch < 1:
+            raise ValueError("max_batch must be >= 1")
+        imgs = [np.asarray(a) for a in raw_images]
+        for i, a in enumerate(imgs):
+            if a.dtype != np.uint8 or a.ndim != 3 or a.shape[2] != 3 or a.shape[0] < 1 or a.shape[1] < 1:
+                raise ValueError(f"raw_images[{i}]: expected a uint8 [h, w, 3] BGR image, got {a.dtype} {a.shape}")
+        dev = next(self.parameters()).device
+        if dev.type != "cuda":
+            raise RuntimeError("DepthAnythingV2 (B200 path) needs CUDA parameters: there is no CPU fallback")
+        # every output in one fp32 buffer; pack_layout places [h, w, 4]-byte maps at 16-byte boundaries
+        rows_out, end = ops.pack_layout([(a.shape[0], a.shape[1], 4) for a in imgs])
+        out = torch.empty((end + 3) // 4, dtype=torch.float32, device=dev)
+        if getattr(self, "_staging", None) is None or self._staging.device != dev:
+            self._staging = ops.Staging(dev)
+        with torch.cuda.device(dev):
+            for H, W, idx in self._chunks([a.shape[:2] for a in imgs], input_size, max_batch):
+                rows_in, n_in = ops.pack_layout([imgs[i].shape for i in idx])
+
+                def fill(host, rows_in=rows_in, idx=idx):
+                    for (o, _, _), i in zip(rows_in, idx):
+                        np.copyto(host[o:o + imgs[i].size].reshape(imgs[i].shape), imgs[i])
+                data, desc = self._staging.upload(n_in, rows_in + [rows_out[i] for i in idx], fill)
+                x = ops.resize_cubic_normalize_batch(data, desc[:len(idx)], H, W)
+                ops.upsample_restore_batch(self.forward(x), desc[len(idx):], out)
+        return [out[o // 4:o // 4 + h * w].view(h, w) for o, h, w in rows_out]
 
 
 def get_model(model_name, **kwargs):

@@ -1,5 +1,6 @@
 """Operator-level wrappers over the C ABI, taking torch CUDA tensors. Used by tests/ and tools/ to check each kernel
-against the matching torch op; the model path (model.py) calls ada_forward directly and does not go through here."""
+against the matching torch op, and by the pre/post-processing around the forward (infer.py, DepthAnythingV2.infer_images);
+the forward itself (model.py) calls ada_forward directly and does not go through here."""
 from __future__ import annotations
 
 import ctypes
@@ -229,6 +230,37 @@ def pack_layout(shapes, start=0):
     return rows, off
 
 
+class Staging:
+    """Reused pinned host buffers for one packed uint8 upload and its int64 [n, 3] descriptor table. A stage waits only
+    for the previous upload from the buffers (its copies may still be reading them), then makes one H2D copy of each on
+    the current stream."""
+
+    def __init__(self, device):
+        self.device = device
+        self._data = None
+        self._desc = None
+        self._uploaded = None    # event after the last upload from the buffers (they are rewritten after it)
+
+    def upload(self, end, rows, fill):
+        """fill(host) writes the packed bytes into `host`, a uint8 numpy array of `end` bytes; rows are the descriptor
+        rows. Returns (data uint8 [end], desc int64 [len(rows), 3]) on the device."""
+        if self._uploaded is not None:
+            self._uploaded.synchronize()
+        if self._data is None or self._data.numel() < end:
+            self._data = torch.empty(end, dtype=torch.uint8, pin_memory=True)
+        if self._desc is None or self._desc.shape[0] < len(rows):
+            self._desc = torch.empty(len(rows), 3, dtype=torch.int64, pin_memory=True)
+        fill(self._data.numpy()[:end])
+        self._desc.numpy()[:len(rows)] = rows
+        data = torch.empty(end, dtype=torch.uint8, device=self.device)
+        desc = torch.empty(len(rows), 3, dtype=torch.int64, device=self.device)
+        data.copy_(self._data[:end], non_blocking=True)
+        desc.copy_(self._desc[:len(rows)], non_blocking=True)
+        self._uploaded = torch.cuda.Event()
+        self._uploaded.record()
+        return data, desc
+
+
 def _desc(src, desc):
     assert src.dtype == torch.uint8 and src.is_contiguous()
     assert desc.dtype == torch.int64 and desc.dim() == 2 and desc.shape[1] == 3 and desc.is_contiguous()
@@ -287,6 +319,27 @@ def blend_seam_batch(raw01, amodal, mask01):
     assert raw01.numel() == amodal.numel() == mask01.numel() == B * H * W
     out = torch.empty(B, H, W, dtype=torch.float32, device=raw01.device)
     _call(raw01, L.load().ada_post_blend_seam_batch, _p(raw01), _p(amodal), _p(mask01), _p(out), B, H, W)
+    return out
+
+
+def resize_cubic_normalize_batch(src_u8, desc, H, W, out=None):
+    """DepthAnythingV2.image2tensor of each 3-channel BGR image of the packed buffer at (H, W), bit-exact (cv2's float64
+    INTER_CUBIC, then the ImageNet normalise in float64) -> fp32 [B,3,H,W]."""
+    B = _desc(src_u8, desc)
+    out = _out(out, (B, 3, H, W), torch.float32, src_u8.device)
+    _call(src_u8, L.load().ada_pre_resize_cubic_normalize_batch, _p(src_u8), _p(desc), B, _p(out), H, W)
+    return out
+
+
+def upsample_restore_batch(depth, out_desc, out):
+    """Bilinear (align_corners=True) of each map of depth [B,H,W] fp32 to its own size, into the fp32 buffer `out`: row b
+    of out_desc (int64 [B, 3] device rows of ada_img_desc) holds map b's byte offset into `out` and its (h, w)."""
+    assert depth.dtype == torch.float32 and depth.dim() == 3 and depth.is_contiguous()
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.device == depth.device
+    assert out_desc.dtype == torch.int64 and out_desc.shape == (depth.shape[0], 3) and out_desc.is_contiguous()
+    assert out_desc.device == depth.device
+    B, H, W = depth.shape
+    _call(depth, L.load().ada_post_upsample_restore_batch, _p(depth), B, H, W, _p(out_desc), _p(out))
     return out
 
 

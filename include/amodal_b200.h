@@ -197,6 +197,16 @@ int ada_post_minmax_normalize_batch(const float* depth, int32_t B, int64_t n, fl
 /* ada_post_blend_seam on each of B maps: raw01, amodal, mask01, out [B,H,W]. */
 int ada_post_blend_seam_batch(const float* raw01, const float* amodal, const float* mask01, float* out, int32_t B,
                               int32_t H, int32_t W, void* stream);
+/* ---- the pre/post-processing of DepthAnythingV2.infer_image (depth_anything_v2_raw/dpt.py:186-222) over a batch.
+ * image2tensor, bit-exact: uint8 BGR HWC images (3-channel rows of desc) -> cvtColor(BGR -> RGB) / 255.0 ->
+ * cv2.resize(..., INTER_CUBIC) in float64 -> ImageNet (x - mean) / std in float64 -> out [B,3,H,W] fp32. */
+int ada_pre_resize_cubic_normalize_batch(const uint8_t* src, const ada_img_desc* desc, int32_t B, float* out_chw,
+                                         int32_t H, int32_t W, void* stream);
+/* F.interpolate(depth[:, None], (h, w), mode="bilinear", align_corners=True) of each map of depth [B,H,W] fp32 to its own
+ * size: row b of out_desc (device) gives map b's output (h, w) = (H0, W0) and its byte offset from `out` (a multiple of
+ * 4). ATen's index math, every operation rounded on its own. */
+int ada_post_upsample_restore_batch(const float* depth, int32_t B, int32_t H, int32_t W, const ada_img_desc* out_desc,
+                                    float* out, void* stream);
 /* ---- per-sample evaluation post-ops of the validation loop on the device (SURVEY.md section 8 row f3;
  * discriminative_trainer.py:542-613). pred [h,w] is resized to the ground-truth size (H,W) by nearest sampling (:542),
  * aligned to depth_obs over visible_mask by least squares (src/util/alignment.py:7-54) and scored against depth_gt + 1e-5
